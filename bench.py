@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--workload arxiv|products|pubmed|cora|molecules]
     python bench.py --impl reference ...        # the CPU oracle timed on the host cores
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's outputs as DIR/<name>.npy
 
 A step = one adapter forward + backward over the workload graph.  Default workload (N = 1) is
 BASELINE.json configs[3], the ogbn-arxiv-shaped graph the metric is quoted on (169,343 nodes,
@@ -27,11 +28,13 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import torch  # noqa: E402
 
 METRIC = "gconv_adapter_fwd_bwd_edges_per_sec"
 UNIT = "edges/s"
+DUMP_BYTES = 64 << 20               # --dump-outputs: upper bound of all arrays written
 
 
 # ---------------------------------------------------------------------------------------------
@@ -47,7 +50,36 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--single-adapter", action="store_true",
                     help="molecules / pubmed: ONE adapter fwd+bwd on the workload's graph instead of the host step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (output, input and parameter gradients; "
+                         "a fixed sample of rows when larger than %d MB) as DIR/<name>.npy" % (DUMP_BYTES >> 20))
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs: single-GPU runs of --impl ours only")
+    return args
+
+
+def sample_rows(t, max_rows):
+    """A copy of t[rows] for a fixed, seeded sample of at most max_rows rows, kept in row order (all rows when they fit)."""
+    if t.size(0) <= max_rows:
+        return t.detach().clone()
+    rows = torch.randperm(t.size(0), generator=torch.Generator().manual_seed(0))[:max_rows].sort().values
+    return t.detach().index_select(0, rows.to(t.device))
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: DIR/<name>.npy per array, float32 or float64, at most DUMP_BYTES in all."""
+    import numpy as np
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    for k, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"--dump-outputs: {k} is {a.dtype}, not float32 / float64")
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def workload(args):
@@ -355,11 +387,15 @@ def run_host_workload(args, lib, dev):
     c0 = time.perf_counter()
     t0.record()
     for i in range(args.steps):
-        step(dev_pool[i % len(dev_pool)])
+        loss = step(dev_pool[i % len(dev_pool)])
     t1.record()
     torch.cuda.synchronize()
     ms_step = max(t0.elapsed_time(t1), 1e3 * (time.perf_counter() - c0)) / args.steps
     launches = lib.gca_launch_count() - l0
+    dumped = None
+    if args.dump_outputs:
+        dumped = {"loss": loss.detach().clone()}
+        dumped.update({"grad_" + k: p.grad.clone() for k, p in host.named_parameters() if p.grad is not None})
     t_end = time.perf_counter() + 1.0
     i = 0
     while time.perf_counter() < t_end:
@@ -446,6 +482,8 @@ def run_host_workload(args, lib, dev):
         "cpu_baseline": None,
     }
     GLOBAL_GRAPH_CACHE.clear()
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     print(json.dumps(line))
 
 
@@ -477,6 +515,7 @@ def run_ours(args):
     gd = g_out.to(dev)
     graph = m.graph_for(eid, n)                 # built once; the timed steps reuse it (static graph)
     e_prime = graph.nnz
+    holder = {}
 
     def step():
         xd.grad = None
@@ -484,6 +523,7 @@ def run_ours(args):
             p.grad = None
         y = m(xd, eid)
         y.backward(gd)
+        holder["y"] = y.detach()                # what a caller receives, kept for --dump-outputs (warm-up included)
 
     for _ in range(max(args.warmup, 3)):
         step()
@@ -500,6 +540,11 @@ def run_ours(args):
     torch.cuda.synchronize()
     ms_step = t0.elapsed_time(t1) / args.steps
     launches = lib.gca_launch_count() - l0
+    dumped = None
+    if args.dump_outputs:
+        rows = (DUMP_BYTES // 2) // (2 * 4 * d)     # Y and gX share half the budget; the parameter gradients are small
+        dumped = {"y": sample_rows(holder["y"], rows), "grad_x": sample_rows(xd.grad, rows)}
+        dumped.update({"grad_" + k: p.grad.clone() for k, p in m.named_parameters()})
     # keep the GPU under the same load for ~1 s so nvidia-smi (100 ms period) sees the clocks of this kernel mix
     t_end = time.perf_counter() + 1.0
     while time.perf_counter() < t_end:
@@ -672,8 +717,11 @@ def run_ours(args):
                                              "ms_per_step above is bound by Python / autograd dispatch at this size"}
     if args.workload is None and os.environ.get("GCA_BENCH_NO_PRODUCTS", "0") != "1":
         del xd, gd, eid
+        holder.clear()
         torch.cuda.empty_cache()
         line["products"] = products_subrecord(lib, dev)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     print(json.dumps(line))
 
 

@@ -35,22 +35,6 @@ def test_oracle_restatement_matches_reference_vectors(path):
     assert torch.allclose(b.grad, g["rel_gb"], rtol=1e-6, atol=1e-6)
 
 
-@pytest.mark.skipif(not backbone_ref.reference_available(), reason="/root/reference is only present in the build container")
-def test_oracle_matches_the_reference_functions_live():
-    ref_gcn, ref_rel = backbone_ref.load_reference_functions()
-    torch.manual_seed(3)
-    n = 120
-    ei = torch.randint(0, n, (2, 500))
-    ei = torch.cat([ei, ei.flip(0), torch.arange(n).repeat(2, 1)], dim=1)
-    x = torch.randn(n, 3, 16)
-    assert torch.equal(ref_gcn(x, ei, None), backbone_ref.gcn_conv(x, ei))
-    w = torch.rand(ei.shape[1])
-    assert torch.equal(ref_gcn(x, ei, w), backbone_ref.gcn_conv(x, ei, w))
-    b = torch.randn(3)
-    for trans in ("sigmoid", "identity"):
-        assert torch.equal(ref_rel(x.unsqueeze(0), ei, b, trans), backbone_ref.add_conv_relational_bias(x.unsqueeze(0), ei, b, trans))
-
-
 def test_propagation_equals_the_adapter_normalisation_on_self_looped_graphs():
     """The precondition the CUDA path relies on: with one self loop per node the reference's matrix is D^-1/2 A' D^-1/2
     of the adapter (oracle.pyg_restated.gcn_norm), up to the rounding of sqrt(1/d) vs d^-1/2."""

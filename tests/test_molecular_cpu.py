@@ -50,25 +50,6 @@ def test_oracle_restatement_matches_reference_vectors(path, tag):
             assert torch.allclose(p.grad, want, rtol=1e-5, atol=1e-5 * float(want.abs().max())), k
 
 
-@pytest.mark.skipif(not molecular_ref.reference_available(), reason="/root/reference is only present in the build container")
-def test_oracle_matches_the_reference_classes_live():
-    from gconv_adapter_b200.graphs.synthetic import molecule_batch
-    gin_cls, gcn_cls = molecular_ref.load_reference_classes()
-    ei, _, n = molecule_batch(batch_size=5, seed=9)
-    gen = torch.Generator().manual_seed(1)
-    ea = torch.stack([torch.randint(0, 4, (ei.size(1),), generator=gen), torch.randint(0, 3, (ei.size(1),), generator=gen)], 1)
-    x = torch.randn(n, 16, generator=gen)
-    for ref_cls, ours_cls in ((gin_cls, molecular_ref.MolecularGINConvRef), (gcn_cls, molecular_ref.MolecularGCNConvRef)):
-        torch.manual_seed(3)
-        a = ref_cls(16)
-        torch.manual_seed(3)
-        b = ours_cls(16)
-        assert list(a.state_dict()) == list(b.state_dict())
-        for (ka, va), (kb, vb) in zip(a.state_dict().items(), b.state_dict().items()):
-            assert torch.equal(va, vb), ka
-        assert torch.equal(a(x, ei, ea), b(x, ei, ea))
-
-
 def test_histogram_identity_behind_the_cuda_layers():
     """sum_e emb(type_e) + emb(dir_e) over the incoming edges of a node == counts[node] @ tables (self loop = type 4, dir 0)."""
     from gconv_adapter_b200.graphs.synthetic import molecule_batch
