@@ -65,6 +65,26 @@ def _align(nbytes: int) -> int:
     return (nbytes + 255) // 256 * 256
 
 
+def row_pitch(t: torch.Tensor) -> int:
+    """Row pitch (elements) to pass with a ``[n, d]`` operand that ``kernel_operand`` accepted.  A single row has no
+    pitch: PyTorch calls a ``[1, d]`` tensor with unit inner stride contiguous whatever its stride(0) (``x.t()`` of a
+    ``[d, 1]`` tensor has strides ``(1, 1)``), so ``d`` is passed, which the kernels accept."""
+    return t.shape[1] if t.shape[0] <= 1 else t.stride(0)
+
+
+def kernel_operand(t: torch.Tensor) -> tuple[torch.Tensor, int]:
+    """``(t, pitch)`` when the kernels can read or write the ``[n, d]`` fp32 tensor ``t`` in place: unit inner stride,
+    row pitch >= d and a multiple of 4 elements, base 16 B aligned (include/gca.h).  Otherwise a dense copy and ``d``.
+    Column windows of wider tensors and gradients of ``torch.cat`` outputs pass as they are; broadcast gradients
+    (stride 0, e.g. of ``y.sum(0)``), odd pitches and misaligned views are copied."""
+    n, d = t.shape
+    if t.stride(-1) == 1 and t.data_ptr() % 16 == 0:
+        ld = row_pitch(t)
+        if ld >= d and ld % 4 == 0:
+            return t, ld
+    return t.clone(memory_format=torch.contiguous_format), d
+
+
 class _GConvAdapterFunction(torch.autograd.Function):
     """Y = s * (Ahat act(Ahat X Wd^T + bd) Wu^T + bu [+ X]) and its gradients, one graph handle.
 
@@ -74,6 +94,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, w_down, b_down, w_up, b_up, scalar, graph: GraphStructure, act: int, skip: bool):
         lib = _cabi.load()
+        x, ldx = kernel_operand(x)
         n, d = x.shape
         r = w_down.shape[0]
         dev = x.device
@@ -93,7 +114,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
         zp_ptr, h2_ptr = base, base + rw
         h1_ptr = base + 2 * rw if silu else None
         ws_ptr = base + (3 if silu else 2) * rw
-        _cabi.check(lib.gca_forward(graph.handle, x.data_ptr(), x.stride(0), w_down.data_ptr(), b_down.data_ptr(),
+        _cabi.check(lib.gca_forward(graph.handle, x.data_ptr(), ldx, w_down.data_ptr(), b_down.data_ptr(),
                                     w_up.data_ptr(), b_up.data_ptr(), _ptr(scalar), act, int(skip), ws_ptr,
                                     zp_ptr, h1_ptr, h2_ptr, y.data_ptr(), y.stride(0), d, r, stream), "gca_forward")
         ctx.graph, ctx.act, ctx.skip = graph, act, skip
@@ -119,8 +140,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
         n, d = x.shape
         r = w_down.shape[0]
         dev = x.device
-        if g_y.stride(-1) != 1 or g_y.stride(0) % 4 != 0 or g_y.data_ptr() % 16 != 0:
-            g_y = g_y.contiguous()
+        g_y, ldg = kernel_operand(g_y)
         stream = _raw_stream(dev)
         rw = ctx.rw
         base = buf.data_ptr()
@@ -136,7 +156,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
         g_bd = torch.empty((r,), dtype=torch.float32, device=dev)
         g_s = torch.empty((1,), dtype=torch.float32, device=dev) if scalar is not None else None
         ws = torch.empty(_sizes(lib, ctx.graph, d, r)[1], dtype=torch.uint8, device=dev)
-        _cabi.check(lib.gca_backward(ctx.graph.handle, g_y.data_ptr(), g_y.stride(0), x.data_ptr(), x.stride(0),
+        _cabi.check(lib.gca_backward(ctx.graph.handle, g_y.data_ptr(), ldg, x.data_ptr(), row_pitch(x),
                                      zp_ptr, h1_ptr, h2_ptr, w_down.data_ptr(), w_up.data_ptr(),
                                      b_up.data_ptr(), _ptr(scalar), ctx.act, int(ctx.skip), ws.data_ptr(),
                                      _ptr(g_x), g_x.stride(0) if need_x else d, g_wd.data_ptr(), g_bd.data_ptr(),
@@ -151,8 +171,7 @@ class _LayerNormScaleFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias, scalar, eps: float):
         lib = _cabi.load()
-        if x.stride(-1) != 1 or x.stride(0) % 4 != 0 or x.data_ptr() % 16 != 0:
-            x = x.contiguous()
+        x, ldx = kernel_operand(x)
         n, d = x.shape
         dev = x.device
         stream = _raw_stream(dev)
@@ -160,7 +179,7 @@ class _LayerNormScaleFunction(torch.autograd.Function):
         stats = torch.empty((2, max(n, 1)), dtype=torch.float32, device=dev)
         weight = weight.contiguous() if weight is not None else None
         bias = bias.contiguous() if bias is not None else None
-        _cabi.check(lib.gca_layernorm_scale_fwd(x.data_ptr(), x.stride(0), _ptr(weight), _ptr(bias), _ptr(scalar), float(eps),
+        _cabi.check(lib.gca_layernorm_scale_fwd(x.data_ptr(), ldx, _ptr(weight), _ptr(bias), _ptr(scalar), float(eps),
                                                 y.data_ptr(), y.stride(0), stats[0].data_ptr(), stats[1].data_ptr(), n, d,
                                                 stream), "gca_layernorm_scale_fwd")
         ctx.has = (weight is not None, bias is not None, scalar is not None)
@@ -178,15 +197,14 @@ class _LayerNormScaleFunction(torch.autograd.Function):
         scalar = rest.pop(0) if ctx.has[2] else None
         n, d = x.shape
         dev = x.device
-        if g_y.stride(-1) != 1 or g_y.stride(0) % 4 != 0 or g_y.data_ptr() % 16 != 0:
-            g_y = g_y.contiguous()
+        g_y, ldg = kernel_operand(g_y)
         stream = _raw_stream(dev)
         g_x = torch.empty((n, d), dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
         g_w = torch.empty((d,), dtype=torch.float32, device=dev) if weight is not None else None
         g_b = torch.empty((d,), dtype=torch.float32, device=dev) if bias is not None else None
         g_s = torch.empty((1,), dtype=torch.float32, device=dev) if scalar is not None else None
         ws = torch.empty(lib.gca_layernorm_scratch_bytes(d), dtype=torch.uint8, device=dev)
-        _cabi.check(lib.gca_layernorm_scale_bwd(g_y.data_ptr(), g_y.stride(0), x.data_ptr(), x.stride(0), _ptr(weight),
+        _cabi.check(lib.gca_layernorm_scale_bwd(g_y.data_ptr(), ldg, x.data_ptr(), row_pitch(x), _ptr(weight),
                                                 _ptr(bias), _ptr(scalar), stats[0].data_ptr(), stats[1].data_ptr(), _ptr(g_x),
                                                 g_x.stride(0) if g_x is not None else d, _ptr(g_w), _ptr(g_b), _ptr(g_s),
                                                 ws.data_ptr(), n, d, stream), "gca_layernorm_scale_bwd")
@@ -345,8 +363,6 @@ class GConvAdapter(nn.Module):
         dp, wd, bd, wu, bu = self._padded_params(d, self.bottleneck_size)
         if dp != d:
             x2 = F.pad(x2, (0, dp - d))
-        if x2.stride(-1) != 1 or x2.stride(0) % 4 != 0 or x2.data_ptr() % 16 != 0:
-            x2 = x2.contiguous()
         graph = self.graph_for(edge_index, n)
         fused_scalar = self.scalar if self.normalization is None else None
         out = _GConvAdapterFunction.apply(x2, wd, bd, wu, bu, fused_scalar, graph, self._act, self.skip_connection)

@@ -39,7 +39,7 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from . import _cabi
-from .finetune.gconv_adapter import GConvAdapter
+from .finetune.gconv_adapter import GConvAdapter, kernel_operand, row_pitch
 from .graphs.csr import GraphStructure
 
 
@@ -87,7 +87,7 @@ class CudaPhases:
 
     def fwd_project(self, g, x, wd, out_local, push=None):
         d, r = x.shape[1], wd.shape[0]
-        _cabi.check(self.lib.gca_fwd_project(g.handle, x.data_ptr(), x.stride(0), wd.data_ptr(), out_local.data_ptr(),
+        _cabi.check(self.lib.gca_fwd_project(g.handle, x.data_ptr(), row_pitch(x), wd.data_ptr(), out_local.data_ptr(),
                                              self._push(push), d, r, self._stream(x)), "gca_fwd_project")
 
     def fwd_hop1(self, g, p_full, bd, act, z_local, h1_local, hub=None, push=None):
@@ -97,7 +97,7 @@ class CudaPhases:
 
     def fwd_hop2_up(self, g, z_full, x, wu, bu, scalar, skip, h2_local, y, hub=None):
         d, r = wu.shape
-        _cabi.check(self.lib.gca_fwd_hop2_up(g.handle, z_full.data_ptr(), x.data_ptr(), x.stride(0), wu.data_ptr(),
+        _cabi.check(self.lib.gca_fwd_hop2_up(g.handle, z_full.data_ptr(), x.data_ptr(), row_pitch(x), wu.data_ptr(),
                                              bu.data_ptr(), _ptr(scalar), int(skip), h2_local.data_ptr(), y.data_ptr(),
                                              y.stride(0), _ptr(hub), d, r, self._stream(x)), "gca_fwd_hop2_up")
 
@@ -106,7 +106,7 @@ class CudaPhases:
 
     def bwd_up(self, g, gy, h2_local, wu, scalar, gh2_local, scratch, push=None):
         d, r = wu.shape
-        _cabi.check(self.lib.gca_bwd_up(g.handle, gy.data_ptr(), gy.stride(0), h2_local.data_ptr(), wu.data_ptr(),
+        _cabi.check(self.lib.gca_bwd_up(g.handle, gy.data_ptr(), row_pitch(gy), h2_local.data_ptr(), wu.data_ptr(),
                                         _ptr(scalar), gh2_local.data_ptr(), scratch.data_ptr(), self._push(push), d, r,
                                         self._stream(gy)), "gca_bwd_up")
 
@@ -118,8 +118,8 @@ class CudaPhases:
 
     def bwd_hop1_down(self, g, gh1_full, x, gy, wd, scalar, skip, gp_local, gx, scratch, hub=None):
         r, d = wd.shape
-        _cabi.check(self.lib.gca_bwd_hop1_down(g.handle, gh1_full.data_ptr(), x.data_ptr(), x.stride(0), gy.data_ptr(),
-                                               gy.stride(0), wd.data_ptr(), _ptr(scalar), int(skip), gp_local.data_ptr(),
+        _cabi.check(self.lib.gca_bwd_hop1_down(g.handle, gh1_full.data_ptr(), x.data_ptr(), row_pitch(x), gy.data_ptr(),
+                                               row_pitch(gy), wd.data_ptr(), _ptr(scalar), int(skip), gp_local.data_ptr(),
                                                _ptr(gx), gx.stride(0) if gx is not None else d, scratch.data_ptr(),
                                                _ptr(hub), d, r, self._stream(x)), "gca_bwd_hop1_down")
 
@@ -246,7 +246,7 @@ class _PartitionedFunction(torch.autograd.Function):
         world, s, lo, n, d, r = ctx.meta
         backend, graph, comm = ctx.backend, ctx.graph, ctx.comm
         dev = x.device
-        g_y = g_y.contiguous()
+        g_y, _ = kernel_operand(g_y)
         bufs = comm.buffers(world * s, r, dev, ("gh2", "gh1"))
         gh2_full, gh1_full = bufs["gh2"], bufs["gh1"]
         gp = torch.empty((max(n + (n & 1), 2), r), dtype=torch.float32, device=dev)     # even row count (gca_bwd_hop1_down)
@@ -420,7 +420,7 @@ class PartitionedGConvAdapter(GConvAdapter):
             raise RuntimeError("PartitionedGConvAdapter needs hidden % 4 == 0 and bottleneck in {8,16,32,64}")
         graph = self._graph(edge_index, num_nodes, lo, hi)
         comm = self._get_comm(num_nodes, x_local.device)
-        x_local = x_local.contiguous()
+        x_local, _ = kernel_operand(x_local)
         fused_scalar = self.scalar if self.normalization is None else None
         out = _PartitionedFunction.apply(x_local, self.conv_down.lin.weight, self.conv_down.bias,
                                          self.conv_up.lin.weight, self.conv_up.bias, fused_scalar, graph, self._act,

@@ -14,7 +14,9 @@
  *  - every call is asynchronous on `stream` (a cudaStream_t) except where noted; nothing
  *    is allocated by the library: the caller passes workspaces sized by the *_bytes calls.
  *  - return value: GCA_OK (0) or a negative gca_status; no exceptions cross the ABI.
- *  - fp32 row-major tensors; `ld*` is the row pitch in elements (>= d, multiple of 4).
+ *  - fp32 row-major tensors; `ld*` is the row pitch in elements (>= d, multiple of 4).  X / Y / gY / gX pointers
+ *    (and every other pitched operand) are 16 B aligned: the kernels load and store them as float4 and through tensor
+ *    maps, and do not check.  A column window of a wider tensor qualifies when its first column is.
  *  - re-entrant per (graph handle, stream): a built handle is read-only; every byte a call scribbles on (projection
  *    scratch, partial sums, the partial sums of hub rows) comes from the caller's per-call workspaces, so one handle
  *    may serve several streams / threads / adapters at once (SURVEY.md section 8b "Threading").
