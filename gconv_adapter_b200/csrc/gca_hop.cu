@@ -150,9 +150,8 @@ int launch_hop_t(const Csr& c, const float* F, const float* bias, int act,
     int grid = (n + 8 * GPW - 1) / (8 * GPW);
     // one resident wave: the warps loop over their row batches; a second, partially filled wave of CTAs only adds a tail
     static const int per_sm = [] {
-        const char* e = getenv("GCA_HOP_CTAS");
-        int v = e ? atoi(e) : 0;
-        if (v <= 0 && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, k_hop<R, BWD>, 256, 0) != cudaSuccess) v = 0;
+        int v = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, k_hop<R, BWD>, 256, 0) != cudaSuccess) v = 0;
         return v > 0 && v <= 16 ? v : 8;
     }();
     const int cap = BWD ? (kMaxPartsBd < per_sm * num_sms() ? kMaxPartsBd : per_sm * num_sms()) : per_sm * num_sms();

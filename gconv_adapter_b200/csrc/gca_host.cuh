@@ -89,6 +89,7 @@ bool get_box_map(CUtensorMap* tm, const float* base, int rows, int cols, int64_t
 // K1: out[i, 0:r] = rowscale[i] * s * sum_k A[i,k] W[k, 0:r]    (w_is_rd: W stored [r, d], else [d, r])
 int launch_project(int r, bool w_is_rd, const float* A, int64_t lda, const float* W, const float* rowscale, const float* scalar,
                    float* out, int n, int d, cudaStream_t st);
+// K1 on tcgen05 / TMEM (gca_tc_project.cu): r = 32 only, GCA_ERR_UNSUPPORTED otherwise
 int launch_project_tc(int r, bool w_is_rd, const float* A, int64_t lda, const float* W, const float* rowscale,
                       const float* scalar, float* out, int n, int d, cudaStream_t st);
 // K2: r-wide hop (forward: bias + act ; backward: act' + bias-gradient partials ; plain: just the hop)

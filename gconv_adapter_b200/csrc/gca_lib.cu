@@ -44,7 +44,6 @@ static bool env_flag(const char* name) {
 //   GCA_DISABLE_TMA=1     behave as if the driver refused every tensor map (kernels that need none take over)
 //   GCA_DISABLE_PDL=1     every kernel fully serialised (no programmatic dependent launch)
 //   GCA_SPLIT_MB=<n>      gathered operand above n MB: K3 = plain hop + expand-only (default 160)
-//   GCA_STREAM_TF32=1     streaming family with 3xTF32 products instead of the scaled 2xFP16 split
 //   GCA_DISABLE_BWD_FUSE=1  backward tail as K3 (hop + expand) + K4 (weight gradient) instead of the one-pass kernel
 bool tc_enabled() { static const bool on = !env_flag("GCA_DISABLE_TC"); return on; }
 bool stream_enabled() { static const bool on = !env_flag("GCA_DISABLE_STREAM"); return on; }

@@ -8,32 +8,38 @@
 // active - every LDG of a warp shares one scoreboard, so a warp never overlaps its own loads with its tensor-core work
 // (profiles/README.md section 2b) - and the backward read gY once for the projection and once more for the weight
 // gradient.  Here the copy engine streams [32 rows x d] tiles into a shared-memory ring (tensor-map boxes of
-// 32 x 32 fp32, SWIZZLE_128B, mbarrier hand-over) and warp-specialised consumers read every tile from shared memory:
+// 32 x 32 fp32, SWIZZLE_128B, mbarrier hand-over) and warp-specialised consumers read every tile from shared memory.
+// Warp 0 is the producer in every layout: one thread issues the boxes of tile k + stages - 1 as soon as all consumers
+// released the stage.  The consumers come in three layouts:
 //
-//   warp 0        producer: one thread issues the boxes of tile k + stages - 1 as soon as all consumers released the stage
-//   warps 1-8     projection (if PROJ): warp w owns the 32-column box w of every tile (W fragments for those 32 k's
-//                 live in registers, split into tf32 hi / lo once), multiplies both 16-row m-tiles of the tile and
-//                 leaves a [32, R] partial in one of two shared-memory buffers (mbarrier red_full / red_free).
-//                 The tile's 32 row scales arrive with the tile (1D bulk copy into the stage) and are applied here.
-//   warps 9-10    projection epilogue (if PROJ): add the eight partials of a tile in box order and store the rows -
-//                 the MMA warps never wait for it unless they run two tiles ahead.  (No global load anywhere in the
-//                 consumers: a cold rowscale LDG per tile paced the whole kernel at one DRAM latency per tile.)
-//   next 8 warps  weight gradient (if WGRAD): warp w owns the same box w as the N dimension (32 columns = 4 n-tiles),
-//                 K = the 32 rows of the tile (4 k-steps), M = R.  The H tile [32, R] arrives through its own
-//                 tensor map in the same stage.  Accumulators stay in registers for the whole kernel (folded into a
-//                 running fp32 sum every 4 tiles: the tensor core's accumulator truncates) -> ONE partial per CTA.
+//   projection (PROJ: project_fwd, project_bwd)                                     1 + 8 + 2 warps
+//     warps 1-8     warp w owns the 32-column box w of every tile (W fragments for those 32 k's live in registers, split
+//                   once), multiplies both 16-row m-tiles of the tile and leaves a [32, R] partial in one of two
+//                   shared-memory buffers (mbarrier red_full / red_free).  The tile's 32 row scales arrive with the tile
+//                   (1D bulk copy into the stage) and are applied here.
+//     warps 9-10    epilogue: add the eight partials of a tile in box order and store the rows - the MMA warps never
+//                   wait for it unless they run two tiles ahead.  (No global load anywhere in the consumers: a cold
+//                   rowscale LDG per tile paced the whole kernel at one DRAM latency per tile.)
+//   fused (PROJ + WGRAD: bwd_up at r = 16)                                          1 + 16 + 2 warps
+//     warps 1-16    warp (w, mt) owns the 16-row m-tile mt of box w: the projection of those rows as above, and the
+//                   weight gradient over the same rows from the same converted fragments (see the role below).
+//     warps 17-18   the projection epilogue.
+//   weight gradient (WGRAD, + DOT: wgrad_up, wgrad_down)                            1 + 8 warps
+//     warps 1-8     warp w owns box w as the N dimension (32 columns = 4 n-tiles), K = the 32 rows of the tile (2 k16
+//                   steps), M = R.  The H tile [32, R] arrives through its own tensor map in the same stage.
+//                   Accumulators stay in registers for the whole kernel (unscaled into a running fp32 sum every tile)
+//                   -> ONE partial per CTA.
 //
 // Fragment reads are bank-conflict free by construction (g = lane >> 2, t = lane & 3):
 //   projection A-fragment: LDS.128 of chunk 4*kb2 + t of rows pg(g) and pg(g) + 8 with pg(g) = (g >> 1) + 4 (g & 1):
 //       a quarter warp (g in {2q, 2q+1}) touches rows q and q + 4, whose swizzle XORs differ in bit 2.
-//       One float4 feeds two k-steps through the K permutation  k-step s: k = t -> column 4t + 2s, k = t + 4 -> 4t + 2s + 1.
-//   weight-gradient B-fragment: LDS.128 of chunk g of rows 8 ks + {0,3,4,7}[t] (b0) and 8 ks + {1,2,5,6}[t] (b1); the
-//       float4 feeds the four n-tiles through the column permutation  col = 32 w + 4 n + j  (n-tile j).
-// 3xTF32 as everywhere: x = hi + lo, A B ~= A_hi B_hi + A_lo B_hi + A_hi B_lo (error ~2^-21 per product).
+//       One float4 feeds one k16 step through the K permutation  k = 2t, 2t+1 -> column 4t, 4t+1 ; k = 2t+8, 2t+9 -> 4t+2, 4t+3.
+//   weight-gradient B-fragment: LDS.128 of chunk g of rows 16 ks2 + {0,3,4,7}[t] (+ 8) (k = 2t, k = 2t+8) and
+//       16 ks2 + {1,2,5,6}[t] (+ 8) (k = 2t+1, 2t+9); the float4 feeds the four n-tiles through the column permutation
+//       col = 32 w + 4 n + j  (n-tile j).
+// Arithmetic: the scaled 2xFP16 split of gca_stream.cuh, three m16n8k16 per product.
 //
 // Reference semantics: the two Linear layers of /root/reference/src/finetune/gconv_adapter.py:92 and their autograd.
-#include <cstdlib>
-
 #include "gca_common.cuh"
 #include "gca_device.cuh"
 #include "gca_host.cuh"
@@ -45,16 +51,20 @@ namespace {
 constexpr int kSRows = 32;                 // rows per tile
 constexpr int kSBox = 32 * kSRows * 4;     // one 32-column box of a tile: 4 KB, SWIZZLE_128B
 constexpr int kSWarps = 8;                 // consumer warps per role = column boxes of a 256-wide tile
-constexpr int kSFold = 4;                  // tiles between two folds of the tensor-core accumulators
 constexpr int kSEpi = 2;                   // epilogue warps of the projection role
 
-// MMA warps per box of the projection role (two - one 16-row m-tile each - measured no faster than one: 43.7 vs 44.0 us)
-__host__ __device__ constexpr int proj_split(int r, bool proj, bool wgrad) { return (void)r, (void)proj, (void)wgrad, 1; }
-// PROJ + WGRAD with the fp16 split runs both on ONE set of warps ("fused role", see k_dense_stream)
-__host__ __device__ constexpr bool fused_role(bool proj, bool wgrad, bool f16) { return proj && wgrad && f16; }
-__host__ __device__ constexpr int stream_threads(int r, bool proj, bool wgrad, bool f16) {
-    return fused_role(proj, wgrad, f16) ? 32 * (1 + 2 * kSWarps + kSEpi)
-                                        : 32 * (1 + (proj ? kSWarps * proj_split(r, proj, wgrad) + kSEpi : 0) + (wgrad ? kSWarps : 0));
+// warps that read the stages: one per (box, m-tile) in the fused layout, else one per box
+__host__ __device__ constexpr int stream_consumers(bool proj, bool wgrad) { return proj && wgrad ? 2 * kSWarps : kSWarps; }
+// producer + consumers + the projection epilogue
+__host__ __device__ constexpr int stream_threads(bool proj, bool wgrad) {
+    return 32 * (1 + stream_consumers(proj, wgrad) + (proj ? kSEpi : 0));
+}
+
+// element (row, c) of the [32, R] H tile of a stage: 128-byte swizzled rows at r = 32, plain rows at r = 16
+template <int R>
+__device__ __forceinline__ float hload(const uint8_t* ht, int row, int c) {
+    if (R == 32) return *reinterpret_cast<const float*>(ht + box_off(row, c >> 2) + (c & 3) * 4);
+    return *reinterpret_cast<const float*>(ht + (row * R + c) * 4);
 }
 
 struct StreamParams {
@@ -65,27 +75,24 @@ struct StreamParams {
     gca_push push;   // peers that receive every projected row as well (count = 0: none)
 };
 
-template <int R, bool PROJ, bool WGRAD, bool DOT, bool W_IS_RD, bool F16>
-__global__ void __launch_bounds__(stream_threads(R, PROJ, WGRAD, F16), 1)
+template <int R, bool PROJ, bool WGRAD, bool DOT, bool W_IS_RD>
+__global__ void __launch_bounds__(stream_threads(PROJ, WGRAD), 1)
 k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmH, const StreamParams p) {
     constexpr int NT = R / 8, MT = R / 16;
-    constexpr int PW = proj_split(R, PROJ, WGRAD);          // MMA warps per box of the projection role
-    constexpr int kProjWarps = kSWarps * PW;
-    constexpr bool FUSED = fused_role(PROJ, WGRAD, F16);
-    constexpr int kFusedWarps = 2 * kSWarps;              // fused role: (box, m-tile) per warp
-    constexpr int kConsumers = FUSED ? kFusedWarps : (PROJ ? kProjWarps : 0) + (WGRAD ? kSWarps : 0);
+    constexpr bool FUSED = PROJ && WGRAD;
+    constexpr int kConsumers = stream_consumers(PROJ, WGRAD);
     extern __shared__ uint8_t smem_unaligned[];
     uint8_t* smem = smem_unaligned + ((1024u - (smem_addr(smem_unaligned) & 1023u)) & 1023u);
     const uint32_t bar0 = smem_addr(smem + p.bar_off);
     auto full = [&](int s) { return bar0 + 8u * (uint32_t)s; };
     auto empty = [&](int s) { return bar0 + 8u * (uint32_t)(p.stages + s); };
-    auto red_full = [&](int b) { return bar0 + 8u * (uint32_t)(2 * p.stages + b); };        // 8 MMA warps -> epilogue
+    auto red_full = [&](int b) { return bar0 + 8u * (uint32_t)(2 * p.stages + b); };        // MMA warps -> epilogue
     auto red_free = [&](int b) { return bar0 + 8u * (uint32_t)(2 * p.stages + 2 + b); };    // epilogue -> MMA warps
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (threadIdx.x == 0) {
         for (int s = 0; s < p.stages; ++s) { mbar_init(full(s), 1); mbar_init(empty(s), kConsumers); }
-        for (int b = 0; b < 2; ++b) { mbar_init(red_full(b), FUSED ? kFusedWarps : kProjWarps); mbar_init(red_free(b), kSEpi); }
+        for (int b = 0; b < 2; ++b) { mbar_init(red_full(b), kConsumers); mbar_init(red_free(b), kSEpi); }
         mbar_fence_init();
     }
     __syncthreads();
@@ -126,8 +133,8 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int cw = warp - 1;
     const int g = lane >> 2, t = lane & 3;
 
-    if (FUSED && cw < kFusedWarps) {
-        // ===================== fused role (PROJ + WGRAD, fp16 split): one conversion serves both products =====================
+    if (FUSED && cw < kConsumers) {
+        // ===================== fused role (PROJ + WGRAD): one conversion serves both products =====================
         // Warp (w, mt) owns the 16-row m-tile mt of box w of every tile (16 warps: four per scheduler hide each other's
         // shuffle-max -> convert -> HMMA -> movmatrix -> HMMA chains; with 8 warps the same work ran at 27 % issue utilisation).
         // It converts its 16 x 32 half box ONCE into projection A-fragments (fp16 hi / lo, its own power-of-two scale),
@@ -136,7 +143,6 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         // into (rows pg(2t), pg(2t+1) ; column C(g)) = the B-fragment of the weight gradient over the SAME 16 rows
         // (k = rows of m-tile mt, n-tiles 2 kb2 / 2 kb2 + 1 = the even / odd column pairs of the 16-column block kb2).
         // Through the permutations lane (g, t) ends up owning G[c = g (+8)][32 w + 16 kb2 + 4t .. + 3]: a float4.
-        if constexpr (FUSED) {
         const int bx = cw % kSWarps, mt = cw / kSWarps;
         const bool active = bx < p.nb;
         uint32_t wf[2][NT][4];
@@ -179,10 +185,6 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                     for (int i = 0; i < 4; ++i) run[m][a_][b_][i] = 0.f;
         csum[0] = csum[1] = make_float4(0.f, 0.f, 0.f, 0.f);
-        auto hload = [&](const uint8_t* ht, int row, int c) -> float {
-            if (R == 32) return *reinterpret_cast<const float*>(ht + box_off(row, c >> 2) + (c & 3) * 4);
-            return *reinterpret_cast<const float*>(ht + (row * R + c) * 4);
-        };
         int s = 0;
         uint32_t ph = 0;
         for (int k = 0; k < my_tiles; ++k) {
@@ -220,7 +222,7 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                         for (int q = 0; q < 8; ++q) {
                             // q: bit 0 = row t / t + 4 (k = 2t / 2t+1), bit 1 = c + 8, bit 2 = rows + 8 (k + 8)
-                            hv[cm][q] = hload(ht, 16 * mt + 8 * (q >> 2) + t + 4 * (q & 1), 16 * cm + g + 8 * ((q >> 1) & 1));
+                            hv[cm][q] = hload<R>(ht, 16 * mt + 8 * (q >> 2) + t + 4 * (q & 1), 16 * cm + g + 8 * ((q >> 1) & 1));
                             mh = fmaxf(mh, fabsf(hv[cm][q]));
                         }
                     float sx, sh, inv_h;
@@ -316,27 +318,24 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             }
         }
         if (bid == 0 && cw == 0 && lane == 0) p.header[p.slot] = 2 * (int)gridDim.x;
-        }
         return;
     }
 
-    if (!FUSED && PROJ && cw < kProjWarps) {
+    if (PROJ && !WGRAD && cw < kConsumers) {
         // ===================== projection warps =====================
         const int bx = cw % kSWarps;
-        const int mt_lo = PW == 2 ? cw / kSWarps : 0, mt_hi = PW == 2 ? mt_lo + 1 : 2;   // m-tiles of this warp
         const bool active = bx < p.nb;
-        // W fragments of this warp's 32 k's, in registers for the whole kernel.
-        //  tf32: wf[ks][nt] = {hi(k0,c), hi(k1,c), lo(k0,c), lo(k1,c)}, k0 = 32 bx + 16 (ks >> 1) + 4 t + 2 (ks & 1), k1 = k0 + 1
-        //  fp16: wf[kb2][nt] = {hi(c0,c0+1), hi(c0+2,c0+3), lo(c0,c0+1), lo(c0+2,c0+3)} (packed pairs), c0 = 32 bx + 16 kb2 + 4 t,
-        //        scaled by this warp's own power of two (inv_w undoes it); in both cases c = 8 nt + g
-        constexpr int KS = F16 ? 2 : 4;
-        uint32_t wf[KS][NT][4];
+        // W fragments of this warp's 32 k's, in registers for the whole kernel: wf[kb2][nt] = {hi(c0,c0+1), hi(c0+2,c0+3),
+        // lo(c0,c0+1), lo(c0+2,c0+3)} (packed pairs), c0 = 32 bx + 16 kb2 + 4 t, c = 8 nt + g, scaled by this warp's own power
+        // of two (inv_w undoes it).  The fused role loads the same fragments with its own copy of this code: as one shared
+        // helper, ptxas scheduled this role differently.
+        uint32_t wf[2][NT][4];
         float inv_w = 1.f;
         auto wload = [&](int k_, int c) -> float {
             if (!active) return 0.f;
             return W_IS_RD ? __ldg(p.W + (size_t)c * p.d + k_) : __ldg(p.W + (size_t)k_ * R + c);
         };
-        if constexpr (F16) {
+        {
             float wv[2][NT][4];
             float m = 0.f;
 #pragma unroll
@@ -357,16 +356,6 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     split_h2(wv[kb2][nt][0], wv[kb2][nt][1], sw, wf[kb2][nt][0], wf[kb2][nt][2]);
                     split_h2(wv[kb2][nt][2], wv[kb2][nt][3], sw, wf[kb2][nt][1], wf[kb2][nt][3]);
                 }
-        } else {
-#pragma unroll
-            for (int ks = 0; ks < KS; ++ks) {
-                const int k0 = 32 * bx + 16 * (ks >> 1) + 4 * t + 2 * (ks & 1);
-#pragma unroll
-                for (int nt = 0; nt < NT; ++nt) {
-                    split_tf32(wload(k0, nt * 8 + g), wf[ks][nt][0], wf[ks][nt][2]);
-                    split_tf32(wload(k0 + 1, nt * 8 + g), wf[ks][nt][1], wf[ks][nt][3]);
-                }
-            }
         }
         const int pg = (g >> 1) + 4 * (g & 1);
         const float sc_s = p.scalar ? __ldg(p.scalar) : 1.f;
@@ -385,71 +374,39 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                         for (int i = 0; i < 4; ++i) acc[a_][mt][nt][i] = 0.f;
             mbar_wait(full(s), ph);
-            float inv_x = 1.f;                                               // undoes the box scale of the fp16 path
+            float inv_x = 1.f;                                               // undoes the box scale
             if (active) {
                 const uint8_t* box = smem + (size_t)s * p.stage_bytes + bx * kSBox;
-                if constexpr (F16) {
-                    // the whole (half) box first: its largest magnitude fixes the scale
-                    float4 x[2][2][2];                                       // [kb2][mt][row g / g + 8]
-                    float m = 0.f;
+                // the whole box first: its largest magnitude fixes the scale
+                float4 x[2][2][2];                                           // [kb2][mt][row g / g + 8]
+                float m = 0.f;
 #pragma unroll
-                    for (int kb2 = 0; kb2 < 2; ++kb2)
+                for (int kb2 = 0; kb2 < 2; ++kb2)
 #pragma unroll
-                        for (int mt = 0; mt < 2; ++mt) {
-                            if (mt < mt_lo || mt >= mt_hi) continue;
-                            x[kb2][mt][0] = lds4(box + box_off(16 * mt + pg, 4 * kb2 + t));
-                            x[kb2][mt][1] = lds4(box + box_off(16 * mt + pg + 8, 4 * kb2 + t));
-                            m = absmax4(absmax4(m, x[kb2][mt][0]), x[kb2][mt][1]);
-                        }
-                    float sx;
-                    pow2_scale(warp_max(m), sx, inv_x);
+                    for (int mt = 0; mt < 2; ++mt) {
+                        x[kb2][mt][0] = lds4(box + box_off(16 * mt + pg, 4 * kb2 + t));
+                        x[kb2][mt][1] = lds4(box + box_off(16 * mt + pg + 8, 4 * kb2 + t));
+                        m = absmax4(absmax4(m, x[kb2][mt][0]), x[kb2][mt][1]);
+                    }
+                float sx;
+                pow2_scale(warp_max(m), sx, inv_x);
 #pragma unroll
-                    for (int kb2 = 0; kb2 < 2; ++kb2)
+                for (int kb2 = 0; kb2 < 2; ++kb2)
 #pragma unroll
-                        for (int mt = 0; mt < 2; ++mt) {
-                            if (mt < mt_lo || mt >= mt_hi) continue;
-                            // one float4 per row = one k16 step: k = 2t, 2t+1 -> columns 4t, 4t+1 ; k = 2t+8, 2t+9 -> 4t+2, 4t+3
-                            uint32_t ah[4], al[4];
-                            split_h2(x[kb2][mt][0].x, x[kb2][mt][0].y, sx, ah[0], al[0]);
-                            split_h2(x[kb2][mt][1].x, x[kb2][mt][1].y, sx, ah[1], al[1]);
-                            split_h2(x[kb2][mt][0].z, x[kb2][mt][0].w, sx, ah[2], al[2]);
-                            split_h2(x[kb2][mt][1].z, x[kb2][mt][1].w, sx, ah[3], al[3]);
+                    for (int mt = 0; mt < 2; ++mt) {
+                        // one float4 per row = one k16 step: k = 2t, 2t+1 -> columns 4t, 4t+1 ; k = 2t+8, 2t+9 -> 4t+2, 4t+3
+                        uint32_t ah[4], al[4];
+                        split_h2(x[kb2][mt][0].x, x[kb2][mt][0].y, sx, ah[0], al[0]);
+                        split_h2(x[kb2][mt][1].x, x[kb2][mt][1].y, sx, ah[1], al[1]);
+                        split_h2(x[kb2][mt][0].z, x[kb2][mt][0].w, sx, ah[2], al[2]);
+                        split_h2(x[kb2][mt][1].z, x[kb2][mt][1].w, sx, ah[3], al[3]);
 #pragma unroll
-                            for (int nt = 0; nt < NT; ++nt) {
-                                mma_f16(acc[0][mt][nt], ah, wf[kb2][nt][0], wf[kb2][nt][1]);
-                                mma_f16(acc[1][mt][nt], al, wf[kb2][nt][0], wf[kb2][nt][1]);
-                                mma_f16(acc[1][mt][nt], ah, wf[kb2][nt][2], wf[kb2][nt][3]);
-                            }
-                        }
-                } else {
-#pragma unroll
-                    for (int kb2 = 0; kb2 < 2; ++kb2) {
-#pragma unroll
-                        for (int mt = 0; mt < 2; ++mt) {
-                            if (mt < mt_lo || mt >= mt_hi) continue;
-                            const int r_lo = 16 * mt + pg, r_hi = r_lo + 8;
-                            const float4 x0 = lds4(box + box_off(r_lo, 4 * kb2 + t));
-                            const float4 x1 = lds4(box + box_off(r_hi, 4 * kb2 + t));
-                            const float e0[4] = {x0.x, x0.y, x0.z, x0.w};
-                            const float e1[4] = {x1.x, x1.y, x1.z, x1.w};
-#pragma unroll
-                            for (int s2 = 0; s2 < 2; ++s2) {
-                                uint32_t ah[4], al[4];
-                                split_tf32(e0[2 * s2], ah[0], al[0]);        // (row g,   k = t)
-                                split_tf32(e1[2 * s2], ah[1], al[1]);        // (row g+8, k = t)
-                                split_tf32(e0[2 * s2 + 1], ah[2], al[2]);    // (row g,   k = t+4)
-                                split_tf32(e1[2 * s2 + 1], ah[3], al[3]);    // (row g+8, k = t+4)
-                                const int ks = kb2 * 2 + s2;
-#pragma unroll
-                                for (int nt = 0; nt < NT; ++nt) {
-                                    mma_tf32(acc[0][mt][nt], ah, wf[ks][nt][0], wf[ks][nt][1]);
-                                    mma_tf32(acc[1][mt][nt], al, wf[ks][nt][0], wf[ks][nt][1]);
-                                    mma_tf32(acc[1][mt][nt], ah, wf[ks][nt][2], wf[ks][nt][3]);
-                                }
-                            }
+                        for (int nt = 0; nt < NT; ++nt) {
+                            mma_f16(acc[0][mt][nt], ah, wf[kb2][nt][0], wf[kb2][nt][1]);
+                            mma_f16(acc[1][mt][nt], al, wf[kb2][nt][0], wf[kb2][nt][1]);
+                            mma_f16(acc[1][mt][nt], ah, wf[kb2][nt][2], wf[kb2][nt][3]);
                         }
                     }
-                }
             }
             // row scales of this lane's rows (16 mt + pg, + 8), read before the stage is released
             float sc[2][2];
@@ -469,7 +426,7 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
                 for (int nt = 0; nt < NT; ++nt)
-                    if (mt >= mt_lo && mt < mt_hi) mine[(mt * NT + nt) * 32 + lane] =
+                    mine[(mt * NT + nt) * 32 + lane] =
                         make_float4((acc[0][mt][nt][0] + acc[1][mt][nt][0]) * inv_x * sc[mt][0], (acc[0][mt][nt][1] + acc[1][mt][nt][1]) * inv_x * sc[mt][0],
                                     (acc[0][mt][nt][2] + acc[1][mt][nt][2]) * inv_x * sc[mt][1], (acc[0][mt][nt][3] + acc[1][mt][nt][3]) * inv_x * sc[mt][1]);
             __syncwarp();
@@ -479,12 +436,12 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         return;
     }
 
-    if (PROJ && cw < (FUSED ? kFusedWarps : kProjWarps) + kSEpi) {
+    if (PROJ && cw < kConsumers + kSEpi) {
         // ===================== projection epilogue warps =====================
         constexpr int kSlots = 2 * NT * 32;
         constexpr int kPer = kSlots / (kSEpi * 32);                          // fragment slots per thread (2 at r = 16)
         const float4* red = reinterpret_cast<const float4*>(smem + p.red_off);
-        const int th = (cw - (FUSED ? kFusedWarps : kProjWarps)) * 32 + lane;
+        const int th = (cw - kConsumers) * 32 + lane;
         // The summed tile is staged as [32][R] floats (two buffers) so that it leaves as whole rows: the tile is ONE
         // contiguous block of 32 R floats in `out` and in every peer's gathered buffer, written with 512 contiguous bytes
         // per warp instruction (8-byte fragment stores ran the NVLink pushes at a third of that).
@@ -524,9 +481,9 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         return;
     }
 
-    if (WGRAD && !FUSED) {
+    if (WGRAD && !PROJ) {
         // ===================== weight-gradient warps =====================
-        const int bx = PROJ ? cw - kProjWarps - kSEpi : cw;
+        const int bx = cw;
         const bool active = bx < p.nb;
         float acc[MT][4][4], run[MT][4][4];
 #pragma unroll
@@ -537,20 +494,8 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 for (int i = 0; i < 4; ++i) { acc[m][j][i] = 0.f; run[m][j][i] = 0.f; }
         float4 csum = make_float4(0.f, 0.f, 0.f, 0.f);
         float dot = 0.f;
-        const int rA = 4 * (t >> 1) + 3 * (t & 1);          // {0, 3, 4, 7}[t]  -> k = t
-        const int rB = 4 * (t >> 1) + 1 + (t & 1);          // {1, 2, 5, 6}[t]  -> k = t + 4
-        auto hload = [&](const uint8_t* ht, int row, int c) -> float {
-            if (R == 32) return *reinterpret_cast<const float*>(ht + box_off(row, c >> 2) + (c & 3) * 4);   // swizzled 128-byte rows
-            return *reinterpret_cast<const float*>(ht + (row * R + c) * 4);
-        };
-        auto fold = [&]() {
-#pragma unroll
-            for (int m = 0; m < MT; ++m)
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) { run[m][j][i] += acc[m][j][i]; acc[m][j][i] = 0.f; }
-        };
+        const int rA = 4 * (t >> 1) + 3 * (t & 1);          // {0, 3, 4, 7}[t]  -> k = 2t (+ 8)
+        const int rB = 4 * (t >> 1) + 1 + (t & 1);          // {1, 2, 5, 6}[t]  -> k = 2t + 1 (+ 8)
         int s = 0;
         uint32_t ph = 0;
         for (int k = 0; k < my_tiles; ++k) {
@@ -560,115 +505,79 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 const uint8_t* boxA = stg + bx * kSBox;
                 const uint8_t* boxB = stg + p.b_off + bx * kSBox;
                 const uint8_t* ht = stg + p.h_off;
-                if constexpr (F16) {
-                    // the whole box first (its largest magnitude fixes the scale): k16 step ks2 covers rows 16 ks2 .. + 15,
-                    // k = 2t, 2t+1, 2t+8, 2t+9 -> rows rA, rB, 8 + rA, 8 + rB (the same conflict-free row sets as the tf32 path)
-                    float4 v[2][4];
-                    float mb = 0.f;
+                // the whole box first (its largest magnitude fixes the scale): k16 step ks2 covers rows 16 ks2 .. + 15,
+                // k = 2t, 2t+1, 2t+8, 2t+9 -> rows rA, rB, 8 + rA, 8 + rB
+                float4 v[2][4];
+                float mb = 0.f;
 #pragma unroll
-                    for (int ks2 = 0; ks2 < 2; ++ks2)
+                for (int ks2 = 0; ks2 < 2; ++ks2)
 #pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            const int row = 16 * ks2 + 8 * (q >> 1) + ((q & 1) ? rB : rA);
-                            v[ks2][q] = lds4(boxA + box_off(row, g));
-                            mb = absmax4(mb, v[ks2][q]);
-                            if (DOT) {
-                                const float4 w = lds4(boxB + box_off(row, g));
-                                dot = fmaf(v[ks2][q].x, w.x, fmaf(v[ks2][q].y, w.y, fmaf(v[ks2][q].z, w.z, fmaf(v[ks2][q].w, w.w, dot))));
-                            } else {
-                                csum = f4_add(csum, v[ks2][q]);
-                            }
-                        }
-                    float hv[2][MT][8];
-                    float mh = 0.f;
-#pragma unroll
-                    for (int ks2 = 0; ks2 < 2; ++ks2)
-#pragma unroll
-                        for (int m = 0; m < MT; ++m)
-#pragma unroll
-                            for (int q = 0; q < 8; ++q) {
-                                const int row = 16 * ks2 + 8 * (q >> 2) + ((q & 1) ? rB : rA);
-                                hv[ks2][m][q] = hload(ht, row, 16 * m + g + 8 * ((q >> 1) & 1));
-                                mh = fmaxf(mh, fabsf(hv[ks2][m][q]));
-                            }
-                    float sb, inv_b, sh, inv_h;
-                    pow2_scale(warp_max(mb), sb, inv_b);
-                    pow2_scale(warp_max(mh), sh, inv_h);
-#pragma unroll
-                    for (int ks2 = 0; ks2 < 2; ++ks2) {
-                        uint32_t bh0[4], bl0[4], bh1[4], bl1[4];
-                        const float e0[4] = {v[ks2][0].x, v[ks2][0].y, v[ks2][0].z, v[ks2][0].w};
-                        const float e1[4] = {v[ks2][1].x, v[ks2][1].y, v[ks2][1].z, v[ks2][1].w};
-                        const float e2[4] = {v[ks2][2].x, v[ks2][2].y, v[ks2][2].z, v[ks2][2].w};
-                        const float e3[4] = {v[ks2][3].x, v[ks2][3].y, v[ks2][3].z, v[ks2][3].w};
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) {
-                            split_h2(e0[j], e1[j], sb, bh0[j], bl0[j]);          // k = 2t, 2t+1   (n-tile j)
-                            split_h2(e2[j], e3[j], sb, bh1[j], bl1[j]);          // k = 2t+8, 2t+9
-                        }
-#pragma unroll
-                        for (int m = 0; m < MT; ++m) {
-                            uint32_t ah[4], al[4];
-                            split_h2(hv[ks2][m][0], hv[ks2][m][1], sh, ah[0], al[0]);   // c = g,   k = 2t, 2t+1
-                            split_h2(hv[ks2][m][2], hv[ks2][m][3], sh, ah[1], al[1]);   // c = g+8
-                            split_h2(hv[ks2][m][4], hv[ks2][m][5], sh, ah[2], al[2]);   // c = g,   k = 2t+8, 2t+9
-                            split_h2(hv[ks2][m][6], hv[ks2][m][7], sh, ah[3], al[3]);   // c = g+8
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) mma_f16(acc[m][j], ah, bh0[j], bh1[j]);
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) mma_f16(acc[m][j], al, bh0[j], bh1[j]);
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) mma_f16(acc[m][j], ah, bl0[j], bl1[j]);
+                    for (int q = 0; q < 4; ++q) {
+                        const int row = 16 * ks2 + 8 * (q >> 1) + ((q & 1) ? rB : rA);
+                        v[ks2][q] = lds4(boxA + box_off(row, g));
+                        mb = absmax4(mb, v[ks2][q]);
+                        if (DOT) {
+                            const float4 w = lds4(boxB + box_off(row, g));
+                            dot = fmaf(v[ks2][q].x, w.x, fmaf(v[ks2][q].y, w.y, fmaf(v[ks2][q].z, w.z, fmaf(v[ks2][q].w, w.w, dot))));
+                        } else {
+                            csum = f4_add(csum, v[ks2][q]);
                         }
                     }
-                    // the accumulators hold box-scaled x tile-scaled values: unscale and fold every tile
-                    const float f = inv_b * inv_h;
+                float hv[2][MT][8];
+                float mh = 0.f;
+#pragma unroll
+                for (int ks2 = 0; ks2 < 2; ++ks2)
 #pragma unroll
                     for (int m = 0; m < MT; ++m)
 #pragma unroll
-                        for (int j = 0; j < 4; ++j)
+                        for (int q = 0; q < 8; ++q) {
+                            const int row = 16 * ks2 + 8 * (q >> 2) + ((q & 1) ? rB : rA);
+                            hv[ks2][m][q] = hload<R>(ht, row, 16 * m + g + 8 * ((q >> 1) & 1));
+                            mh = fmaxf(mh, fabsf(hv[ks2][m][q]));
+                        }
+                float sb, inv_b, sh, inv_h;
+                pow2_scale(warp_max(mb), sb, inv_b);
+                pow2_scale(warp_max(mh), sh, inv_h);
 #pragma unroll
-                            for (int i = 0; i < 4; ++i) { run[m][j][i] = fmaf(acc[m][j][i], f, run[m][j][i]); acc[m][j][i] = 0.f; }
-                } else {
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {
-                    const int ra = 8 * ks + rA, rb = 8 * ks + rB;
-                    const float4 va = lds4(boxA + box_off(ra, g)), vb = lds4(boxA + box_off(rb, g));
+                for (int ks2 = 0; ks2 < 2; ++ks2) {
                     uint32_t bh0[4], bl0[4], bh1[4], bl1[4];
-                    split_tf32(va.x, bh0[0], bl0[0]); split_tf32(va.y, bh0[1], bl0[1]);
-                    split_tf32(va.z, bh0[2], bl0[2]); split_tf32(va.w, bh0[3], bl0[3]);
-                    split_tf32(vb.x, bh1[0], bl1[0]); split_tf32(vb.y, bh1[1], bl1[1]);
-                    split_tf32(vb.z, bh1[2], bl1[2]); split_tf32(vb.w, bh1[3], bl1[3]);
-                    if (DOT) {
-                        const float4 wa = lds4(boxB + box_off(ra, g)), wb = lds4(boxB + box_off(rb, g));
-                        dot = fmaf(va.x, wa.x, fmaf(va.y, wa.y, fmaf(va.z, wa.z, fmaf(va.w, wa.w, dot))));
-                        dot = fmaf(vb.x, wb.x, fmaf(vb.y, wb.y, fmaf(vb.z, wb.z, fmaf(vb.w, wb.w, dot))));
-                    } else {
-                        csum = f4_add(csum, f4_add(va, vb));
+                    const float e0[4] = {v[ks2][0].x, v[ks2][0].y, v[ks2][0].z, v[ks2][0].w};
+                    const float e1[4] = {v[ks2][1].x, v[ks2][1].y, v[ks2][1].z, v[ks2][1].w};
+                    const float e2[4] = {v[ks2][2].x, v[ks2][2].y, v[ks2][2].z, v[ks2][2].w};
+                    const float e3[4] = {v[ks2][3].x, v[ks2][3].y, v[ks2][3].z, v[ks2][3].w};
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        split_h2(e0[j], e1[j], sb, bh0[j], bl0[j]);          // k = 2t, 2t+1   (n-tile j)
+                        split_h2(e2[j], e3[j], sb, bh1[j], bl1[j]);          // k = 2t+8, 2t+9
                     }
 #pragma unroll
                     for (int m = 0; m < MT; ++m) {
                         uint32_t ah[4], al[4];
-                        split_tf32(hload(ht, ra, 16 * m + g), ah[0], al[0]);        // (c = g,   k = t)
-                        split_tf32(hload(ht, ra, 16 * m + g + 8), ah[1], al[1]);    // (c = g+8, k = t)
-                        split_tf32(hload(ht, rb, 16 * m + g), ah[2], al[2]);        // (c = g,   k = t+4)
-                        split_tf32(hload(ht, rb, 16 * m + g + 8), ah[3], al[3]);    // (c = g+8, k = t+4)
+                        split_h2(hv[ks2][m][0], hv[ks2][m][1], sh, ah[0], al[0]);   // c = g,   k = 2t, 2t+1
+                        split_h2(hv[ks2][m][2], hv[ks2][m][3], sh, ah[1], al[1]);   // c = g+8
+                        split_h2(hv[ks2][m][4], hv[ks2][m][5], sh, ah[2], al[2]);   // c = g,   k = 2t+8, 2t+9
+                        split_h2(hv[ks2][m][6], hv[ks2][m][7], sh, ah[3], al[3]);   // c = g+8
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) mma_tf32(acc[m][j], ah, bh0[j], bh1[j]);
+                        for (int j = 0; j < 4; ++j) mma_f16(acc[m][j], ah, bh0[j], bh1[j]);
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) mma_tf32(acc[m][j], al, bh0[j], bh1[j]);
+                        for (int j = 0; j < 4; ++j) mma_f16(acc[m][j], al, bh0[j], bh1[j]);
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) mma_tf32(acc[m][j], ah, bl0[j], bl1[j]);
+                        for (int j = 0; j < 4; ++j) mma_f16(acc[m][j], ah, bl0[j], bl1[j]);
                     }
                 }
+                // the accumulators hold box-scaled x tile-scaled values: unscale and fold every tile
+                const float f = inv_b * inv_h;
+#pragma unroll
+                for (int m = 0; m < MT; ++m)
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+#pragma unroll
+                        for (int i = 0; i < 4; ++i) { run[m][j][i] = fmaf(acc[m][j][i], f, run[m][j][i]); acc[m][j][i] = 0.f; }
             }
-                }
             __syncwarp();
             if (lane == 0) mbar_arrive(empty(s));
-            if (!F16 && (k % kSFold) == kSFold - 1) fold();
             if (++s == p.stages) { s = 0; ph ^= 1u; }
         }
-        if (!F16) fold();
         // ---- per-CTA partial: lane (g, t) owns rows c = g, g+8 (+16 m) and columns 32 bx + 8t .. + 7 ----
         if (active) {
             float* pgp = p.partG + (size_t)bid * R * p.d;
@@ -710,19 +619,10 @@ k_dense_stream(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 template <int R, bool PROJ, bool WGRAD, bool DOT, bool W_IS_RD>
 int launch_one(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmH, const StreamParams& p, size_t smem,
                int grid, const char* name, cudaStream_t st) {
-    // GCA_STREAM_TF32=1 selects the 3xTF32 products instead of the scaled 2xFP16 split (A/B runs, tests)
-    static const bool tf32 = [] { const char* e = getenv("GCA_STREAM_TF32"); return e && e[0] == '1'; }();
-
-    ProfScope ps(name, st, tf32 ? "stream_tf32" : "stream_f16");
-    if (tf32) {
-        auto kern = k_dense_stream<R, PROJ, WGRAD, DOT, W_IS_RD, false>;
-        GCA_TRY(set_smem(kern, smem));
-        GCA_CUDA(launch_pdl(kern, dim3(grid), dim3(stream_threads(R, PROJ, WGRAD, false)), smem, st, tmA, tmB, tmH, p));
-    } else {
-        auto kern = k_dense_stream<R, PROJ, WGRAD, DOT, W_IS_RD, true>;
-        GCA_TRY(set_smem(kern, smem));
-        GCA_CUDA(launch_pdl(kern, dim3(grid), dim3(stream_threads(R, PROJ, WGRAD, true)), smem, st, tmA, tmB, tmH, p));
-    }
+    ProfScope ps(name, st, "stream_f16");
+    auto kern = k_dense_stream<R, PROJ, WGRAD, DOT, W_IS_RD>;
+    GCA_TRY(set_smem(kern, smem));
+    GCA_CUDA(launch_pdl(kern, dim3(grid), dim3(stream_threads(PROJ, WGRAD)), smem, st, tmA, tmB, tmH, p));
     GCA_LAUNCH_OK();
     return GCA_OK;
 }
@@ -776,10 +676,9 @@ int launch_dense_stream_t(const DenseStreamArgs& a, cudaStream_t st) {
         if (wgrad && !get_box_map(&tmH, a.H, a.n, R, R, R, kSRows, R == 32)) return GCA_ERR_UNSUPPORTED;
         const int ntiles = (a.n + kSRows - 1) / kSRows;
         const int grid = ntiles < num_sms() ? ntiles : num_sms();
-        if (proj && wgrad) {
+        if (proj && wgrad) {                                         // R == 16: r = 32 was turned away above
             if (a.w_is_rd) return GCA_ERR_UNSUPPORTED;               // only the backward pairs the two (W = Wu [d, r])
-            if constexpr (R == 16) return launch_one<R, true, true, false, false>(tmA, tmB, tmH, p, smem, grid, a.prof_name, st);
-            return GCA_ERR_UNSUPPORTED;
+            return launch_one<16, true, true, false, false>(tmA, tmB, tmH, p, smem, grid, a.prof_name, st);
         }
         if (proj)
             return a.w_is_rd ? launch_one<R, true, false, false, true>(tmA, tmB, tmH, p, smem, grid, a.prof_name, st)

@@ -14,7 +14,7 @@ namespace {
 __device__ __forceinline__ uint32_t box_off(int row, int chunk) { return (uint32_t)(row * 128 + ((chunk ^ (row & 7)) << 4)); }
 __device__ __forceinline__ float4 lds4(const uint8_t* p) { return *reinterpret_cast<const float4*>(p); }
 
-// ---- scaled 2xFP16 split (F16 = true) ------------------------------------------------------------------------
+// ---- scaled 2xFP16 split ---------------------------------------------------------------------------------------
 // The legacy tensor path issues an f16 m16n8k16 at the rate of a tf32 m16n8k8 (8.6 clk per sub-core, measured:
 // experiments/mma_rate.cu), i.e. twice the k's per instruction.  fp16 and tf32 carry the same 11 significant bits, so
 //     x * 2^e = h0 + h1,  h0 = fp16_rn(x * 2^e),  h1 = fp16_rn(x * 2^e - h0)         A B ~= A0 B0 + A1 B0 + A0 B1

@@ -282,63 +282,51 @@ k_expand_wgrad(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
     }
 }
 
-template <int R>
-int launch_expand_wgrad_t(const float* X, int64_t ldx, const float* gY, int64_t ldg, const float* gP, const float* Wd,
-                          const float* scalar, float* gX, int64_t ldgx, float* partG, float* partDot, int* header, int slot,
-                          int n, int d, cudaStream_t st) {
-    // r = 32 doubles the tensor-core and conversion work per streamed byte: measured 1.76 ms against 0.87 + 0.78 ms for
-    // K3 + K4 at products size, so only r = 16 takes the one-pass kernel
-    if constexpr (R != 16) {
-        return GCA_ERR_UNSUPPORTED;
-    } else {
-        static const bool tf32 = [] { const char* e = getenv("GCA_STREAM_TF32"); return e && e[0] == '1'; }();
-        static const bool off = [] { const char* e = getenv("GCA_DISABLE_BWD_FUSE"); return e && e[0] == '1'; }();
-        if (!tc_enabled() || !stream_enabled() || tf32 || off) return GCA_ERR_UNSUPPORTED;
-        if (!X || !gY || !gP || !gX || d % 32 != 0 || d > 32 * kXWarps || n < 128 * kXRows) return GCA_ERR_UNSUPPORTED;
-        if ((ldx % 4) || (ldg % 4) || (ldgx % 4)) return GCA_ERR_UNSUPPORTED;
-        for (const void* q : {(const void*)X, (const void*)gY, (const void*)gP, (const void*)gX})
-            if (reinterpret_cast<uintptr_t>(q) % 16) return GCA_ERR_UNSUPPORTED;
-        ExpandParams p{};
-        p.Wd = Wd; p.scalar = scalar; p.partG = partG; p.partDot = partDot; p.header = header; p.slot = slot;
-        p.n = n; p.d = d; p.nb = d / 32; p.want_dot = partDot ? 1 : 0;
-        const uint32_t a_bytes = (uint32_t)p.nb * kXBox, h_bytes = (uint32_t)(kXRows * R * 4);
-        p.gy_off = a_bytes;
-        p.h_off = 2 * a_bytes;
-        p.stage_bytes = (p.h_off + h_bytes + 1023u) & ~1023u;
-        p.tx_bytes = 2 * a_bytes + h_bytes;
-        int stages = (int)((227 * 1024 - 256 - 1024) / p.stage_bytes);
-        if (stages > 8) stages = 8;
-        if (stages < 3) return GCA_ERR_UNSUPPORTED;
-        p.stages = stages;
-        p.bar_off = (uint32_t)stages * p.stage_bytes;
-        const size_t smem = (size_t)p.bar_off + 256 + 1024;
-        CUtensorMap tmX, tmG, tmH, tmO;
-        if (!get_box_map(&tmX, X, n, d, ldx, 32, kXRows, true) || !get_box_map(&tmG, gY, n, d, ldg, 32, kXRows, true) ||
-            !get_box_map(&tmO, gX, n, d, ldgx, 32, kXRows, true))
-            return GCA_ERR_UNSUPPORTED;
-        // gP [n, 16] is read as [ceil(n / 2), 32]: two nodes per 128-byte row (the caller's buffer holds an even number of rows)
-        if (R == 16 ? !get_box_map(&tmH, gP, (n + 1) / 2, 32, 32, 32, kXRows / 2, true)
-                    : !get_box_map(&tmH, gP, n, 32, 32, 32, kXRows, true))
-            return GCA_ERR_UNSUPPORTED;
-        auto kern = k_expand_wgrad<R>;
-        GCA_TRY(set_smem(kern, smem));
-        const int ntiles = (n + kXRows - 1) / kXRows;
-        const int grid = ntiles < num_sms() ? ntiles : num_sms();
-        {
-            ProfScope ps("expand_wgrad_bwd", st, "stream_f16");
-            GCA_CUDA(launch_pdl(kern, dim3(grid), dim3(32 * (1 + kXWarps)), smem, st, tmX, tmG, tmH, tmO, p));
-        }
-        GCA_LAUNCH_OK();
-        return GCA_OK;
-    }
-}
-
 }  // namespace
 
 int launch_expand_wgrad(int r, const float* X, int64_t ldx, const float* gY, int64_t ldg, const float* gP, const float* Wd,
                         const float* scalar, float* gX, int64_t ldgx, float* partG, float* partDot, int* header, int slot,
                         int n, int d, cudaStream_t st) {
-    GCA_DISPATCH_R(r, (launch_expand_wgrad_t<R_>(X, ldx, gY, ldg, gP, Wd, scalar, gX, ldgx, partG, partDot, header, slot, n, d, st)));
+    // r = 32 doubles the tensor-core and conversion work per streamed byte: measured 1.76 ms against 0.87 + 0.78 ms for
+    // K3 + K4 at products size, so only r = 16 takes the one-pass kernel
+    if (r != 16) return GCA_ERR_UNSUPPORTED;
+    constexpr int R = 16;
+    static const bool off = [] { const char* e = getenv("GCA_DISABLE_BWD_FUSE"); return e && e[0] == '1'; }();
+    if (!tc_enabled() || !stream_enabled() || off) return GCA_ERR_UNSUPPORTED;
+    if (!X || !gY || !gP || !gX || d % 32 != 0 || d > 32 * kXWarps || n < 128 * kXRows) return GCA_ERR_UNSUPPORTED;
+    if ((ldx % 4) || (ldg % 4) || (ldgx % 4)) return GCA_ERR_UNSUPPORTED;
+    for (const void* q : {(const void*)X, (const void*)gY, (const void*)gP, (const void*)gX})
+        if (reinterpret_cast<uintptr_t>(q) % 16) return GCA_ERR_UNSUPPORTED;
+    ExpandParams p{};
+    p.Wd = Wd; p.scalar = scalar; p.partG = partG; p.partDot = partDot; p.header = header; p.slot = slot;
+    p.n = n; p.d = d; p.nb = d / 32; p.want_dot = partDot ? 1 : 0;
+    const uint32_t a_bytes = (uint32_t)p.nb * kXBox, h_bytes = (uint32_t)(kXRows * R * 4);
+    p.gy_off = a_bytes;
+    p.h_off = 2 * a_bytes;
+    p.stage_bytes = (p.h_off + h_bytes + 1023u) & ~1023u;
+    p.tx_bytes = 2 * a_bytes + h_bytes;
+    int stages = (int)((227 * 1024 - 256 - 1024) / p.stage_bytes);
+    if (stages > 8) stages = 8;
+    if (stages < 3) return GCA_ERR_UNSUPPORTED;
+    p.stages = stages;
+    p.bar_off = (uint32_t)stages * p.stage_bytes;
+    const size_t smem = (size_t)p.bar_off + 256 + 1024;
+    CUtensorMap tmX, tmG, tmH, tmO;
+    if (!get_box_map(&tmX, X, n, d, ldx, 32, kXRows, true) || !get_box_map(&tmG, gY, n, d, ldg, 32, kXRows, true) ||
+        !get_box_map(&tmO, gX, n, d, ldgx, 32, kXRows, true))
+        return GCA_ERR_UNSUPPORTED;
+    // gP [n, 16] is read as [ceil(n / 2), 32]: two nodes per 128-byte row (the caller's buffer holds an even number of rows)
+    if (!get_box_map(&tmH, gP, (n + 1) / 2, 32, 32, 32, kXRows / 2, true)) return GCA_ERR_UNSUPPORTED;
+    auto kern = k_expand_wgrad<R>;
+    GCA_TRY(set_smem(kern, smem));
+    const int ntiles = (n + kXRows - 1) / kXRows;
+    const int grid = ntiles < num_sms() ? ntiles : num_sms();
+    {
+        ProfScope ps("expand_wgrad_bwd", st, "stream_f16");
+        GCA_CUDA(launch_pdl(kern, dim3(grid), dim3(32 * (1 + kXWarps)), smem, st, tmX, tmG, tmH, tmO, p));
+    }
+    GCA_LAUNCH_OK();
+    return GCA_OK;
 }
 
 }  // namespace gca

@@ -1,4 +1,6 @@
 // K1-tc: out[i, 0:R] = rowscale[i] * s * sum_k A[i,k] W[k, 0:R]  on tcgen05 (3xTF32, fp32 TMEM accumulators).
+// The r = 32 projection whenever the streaming family (gca_stream.cu) does not run: n < 2048, d > 256, tensor maps
+// refused, or the family switched off.  r = 16 takes the mma.sync kernel of gca_project.cu instead.
 //
 // Persistent, warp-specialised CTA (one per SM, 21 warps):
 //   warps 0-15  producers : LDG.128 a [128 rows x 64 cols] chunk of A (4 rows x 128 B per warp instruction,
@@ -17,21 +19,11 @@
 // accumulator group ks % NG, the lo*hi corrections to a separate one, and the epilogue adds them with
 // round-to-nearest.
 #include "gca_common.cuh"
+#include "gca_host.cuh"
 #include "gca_tc.cuh"
 
 namespace gca {
 namespace tc {
-
-#ifdef GCA_TC_DEBUG
-// cycles summed over CTAs: [0] producer wait-empty, [1] producer wait-data+split+STS, [2] producer total,
-// [3] MMA wait-full, [4] MMA issue, [5] MMA wait-tempty, [6] epilogue wait-tfull, [7] epilogue rest, [8] kernel total (warp 0)
-__device__ unsigned long long g_dbg[16];
-#define DBG_T(var) const long long var = clock64()
-#define DBG_ADD(slot, expr) dbg_acc[slot] += (expr)
-#else
-#define DBG_T(var)
-#define DBG_ADD(slot, expr)
-#endif
 
 constexpr int kRows = 128;                 // rows per tile  (UMMA M)
 constexpr int kCols = 64;                  // columns per pipeline stage
@@ -68,10 +60,6 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * nstage + 4);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-#ifdef GCA_TC_DEBUG
-    long long dbg_acc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    const long long dbg_t0 = clock64();
-#endif
 
     // ---- one-time setup ----
     if (threadIdx.x == 0) {
@@ -117,7 +105,6 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
         int pq = 0;                                        // how many times it has been filled
         for (int it = grp; it < total; it += kGroups) {
             float4 v[kPerThread];
-            DBG_T(l0);
 #pragma unroll
             for (int j = 0; j < kPerThread; ++j) {
                 // j -> (column half jc, row quad jr): rows wq*32 + jr*4 + ri, column quads jc*8 + k4i
@@ -125,11 +112,7 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
                 const int row = min(ltile * kRows + wq * 32 + jr * 4 + ri, n - 1);
                 v[j] = ldg4_stream(A + (size_t)row * lda + lch * kCols + jc * 32 + k4i * 4);
             }
-            DBG_T(w0);
-            DBG_ADD(2, w0 - l0);
             mbar_wait(empty_bar(ps), (uint32_t)((pq & 1) ^ 1));
-            DBG_T(w1);
-            DBG_ADD(0, w1 - w0);
             uint8_t* st = stages + (size_t)ps * kStageBytes;
 #pragma unroll
             for (int j = 0; j < kPerThread; ++j) {
@@ -138,18 +121,12 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
                 const uint32_t off = (uint32_t)((jc * 8 + k4i) * kColChunk + (rl >> 3) * 128 + (rl & 7) * 16);
                 float4 hi, lo;
                 split_tf32(v[j], hi, lo);
-#ifndef GCA_TC_SKIP_STS
                 *reinterpret_cast<float4*>(st + off) = hi;
                 *reinterpret_cast<float4*>(st + kHalfBytes + off) = lo;
-#else
-                if (hi.x == 123.456f && lo.y == 3.f) *reinterpret_cast<float4*>(st + off) = hi;
-#endif
             }
             fence_proxy_async();
             __syncwarp();
             if (lane == 0) mbar_arrive(full_bar(ps));
-            DBG_T(w2);
-            DBG_ADD(1, w2 - w1);
             lch += kGroups;
             while (lch >= nchunks) { lch -= nchunks; ltile += gridDim.x; }
             ++pq;
@@ -176,21 +153,12 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
                 const uint32_t d_tmem = tmem_base + (uint32_t)(a * kAccCols);
                 uint64_t bd = b_desc0;
                 for (int ch = 0; ch < nchunks; ++ch) {
-                    DBG_T(m0);
                     mbar_wait(full_bar(s), ph);
                     tc_fence_after();
-                    DBG_T(m1);
-                    DBG_ADD(3, m1 - m0);
                     const uint64_t ad = a_desc0 + (uint64_t)s * (uint64_t)(kStageBytes >> 4);
                     const uint32_t later = ch != 0;
 #pragma unroll
-                    for (int ks = 0; ks < (
-#ifdef GCA_TC_SKIP_MMA
-                        1
-#else
-                        kCols / 8
-#endif
-                        ); ++ks) {
+                    for (int ks = 0; ks < kCols / 8; ++ks) {
                         // group g = ks % NG: columns [g*2R, g*2R+R) = hi*hi, [g*2R+R, (g+1)*2R) = hi*lo
                         umma_tf32(d_tmem + (uint32_t)((ks % NG) * 2 * R), ad + ks * kStepA, bd + ks * kStepB, idesc_cat,
                                   ks >= NG ? 1u : later);
@@ -201,8 +169,6 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
                     umma_commit(empty_bar(s));                       // stage reusable once these MMAs retire
                     if (ch == nchunks - 1) umma_commit(tfull_bar(a)); // accumulators complete
                     if (++s == nstage) { s = 0; ph ^= 1u; }
-                    DBG_T(m2);
-                    DBG_ADD(4, m2 - m1);
                 }
             }
         }
@@ -213,11 +179,8 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
         for (int t = 0; t < my_tiles; ++t) {
             const int a = t & 1;
             const int tile = blockIdx.x + t * gridDim.x;
-            DBG_T(e0);
             mbar_wait(tfull_bar(a), (uint32_t)((t >> 1) & 1));
             tc_fence_after();
-            DBG_T(e1);
-            DBG_ADD(6, e1 - e0);
             const uint32_t tb = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(a * kAccCols);
             float v[R];
 #pragma unroll
@@ -251,14 +214,6 @@ k_project_tc(const float* __restrict__ A, int64_t lda, const float* __restrict__
             }
         }
     }
-#ifdef GCA_TC_DEBUG
-    if (lane == 0) {
-        const long long tot = clock64() - dbg_t0;
-        if (warp == 0) { atomicAdd(&g_dbg[0], dbg_acc[0]); atomicAdd(&g_dbg[1], dbg_acc[1]); atomicAdd(&g_dbg[2], dbg_acc[2]); }
-        if (warp == kProdWarps + 4) { atomicAdd(&g_dbg[3], dbg_acc[3]); atomicAdd(&g_dbg[4], dbg_acc[4]); atomicAdd(&g_dbg[8], tot); }
-        if (warp == kProdWarps) { atomicAdd(&g_dbg[6], dbg_acc[6]); atomicAdd(&g_dbg[7], tot); }
-    }
-#endif
     tc_fence_before();
     __syncthreads();
     if (warp == kProdWarps + 4) {
@@ -276,7 +231,7 @@ int launch_project_tc_impl(const float* A, int64_t lda, const float* W, const fl
     int nstage = (int)((budget - fixed) / kStageBytes);
     if (nstage > 4) nstage = 4;
     const size_t smem = fixed + (size_t)nstage * kStageBytes;
-    GCA_CUDA(cudaFuncSetAttribute(k_project_tc<R, W_IS_RD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GCA_TRY(set_smem(k_project_tc<R, W_IS_RD>, smem));
     const int ntiles = (n + kRows - 1) / kRows;
     const int grid = ntiles < num_sms() ? ntiles : num_sms();
     {
@@ -289,24 +244,12 @@ int launch_project_tc_impl(const float* A, int64_t lda, const float* W, const fl
 
 }  // namespace tc
 
-#ifdef GCA_TC_DEBUG
-extern "C" int gca_debug_counters(unsigned long long* out16, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out16, tc::g_dbg, sizeof(unsigned long long) * 16);
-    if (reset) { unsigned long long z[16] = {0}; cudaMemcpyToSymbol(tc::g_dbg, z, sizeof(z)); }
-    return 0;
-}
-#endif
-
 // Returns GCA_ERR_UNSUPPORTED when the shape is not on the tensor-core path (caller falls back to K1).
 int launch_project_tc(int r, bool w_is_rd, const float* A, int64_t lda, const float* W, const float* rowscale,
                       const float* scalar, float* out, int n, int d, cudaStream_t st) {
-    if (d % tc::kCols != 0 || n < 1) return GCA_ERR_UNSUPPORTED;
-    if (r == 16) return w_is_rd ? tc::launch_project_tc_impl<16, true>(A, lda, W, rowscale, scalar, out, n, d, st)
-                                : tc::launch_project_tc_impl<16, false>(A, lda, W, rowscale, scalar, out, n, d, st);
-    if (r == 32) return w_is_rd ? tc::launch_project_tc_impl<32, true>(A, lda, W, rowscale, scalar, out, n, d, st)
-                                : tc::launch_project_tc_impl<32, false>(A, lda, W, rowscale, scalar, out, n, d, st);
-    return GCA_ERR_UNSUPPORTED;
+    if (r != 32 || d % tc::kCols != 0 || n < 1) return GCA_ERR_UNSUPPORTED;
+    return w_is_rd ? tc::launch_project_tc_impl<32, true>(A, lda, W, rowscale, scalar, out, n, d, st)
+                   : tc::launch_project_tc_impl<32, false>(A, lda, W, rowscale, scalar, out, n, d, st);
 }
 
 }  // namespace gca

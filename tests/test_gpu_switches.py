@@ -13,8 +13,8 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-GCA_VARS = ("GCA_DISABLE_TC", "GCA_DISABLE_STREAM", "GCA_DISABLE_TMA", "GCA_DISABLE_PDL", "GCA_SPLIT_MB", "GCA_STREAM_TF32",
-            "GCA_DISABLE_BWD_FUSE", "GCA_DISABLE_SMALL")
+GCA_VARS = ("GCA_DISABLE_TC", "GCA_DISABLE_STREAM", "GCA_DISABLE_TMA", "GCA_DISABLE_PDL", "GCA_SPLIT_MB", "GCA_DISABLE_BWD_FUSE",
+            "GCA_DISABLE_SMALL")
 
 
 def run_case(case: str, env_over: dict) -> dict:
@@ -34,8 +34,6 @@ SETTINGS = {
                                                     "hop_expand_fwd": "tcgen05", "hop_expand_bwd": "tcgen05"}),
     "split_k3": ({"GCA_SPLIT_MB": "0", "GCA_DISABLE_BWD_FUSE": "1"},
                  {"hop_plain_fwd": "", "expand_fwd": "tcgen05", "hop_plain_bwd": "", "expand_bwd": "tcgen05"}),
-    "stream_tf32": ({"GCA_STREAM_TF32": "1"}, {"project_fwd": "stream_tf32", "bwd_up": "stream_tf32", "wgrad_down": "stream_tf32",
-                                               "hop_expand_bwd": "tcgen05"}),
     "no_stream": ({"GCA_DISABLE_STREAM": "1"}, {"project_fwd": "mma", "project_bwd": "mma", "wgrad_up": "mma", "wgrad_down": "mma",
                                                 "hop_expand_fwd": "tcgen05"}),
     "no_tma": ({"GCA_DISABLE_TMA": "1"}, {"project_fwd": "mma", "wgrad_up": "mma", "hop_expand_fwd": "mma", "hop_expand_bwd": "mma"}),
