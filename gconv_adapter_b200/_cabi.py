@@ -66,6 +66,7 @@ SIGNATURES = {
     "gca_fwd_project": (C.c_int, [_f, _f, _i64, _f, _f, C.POINTER(Push), _i32, _i32, _f]),
     "gca_fwd_hop1": (C.c_int, [_f, _f, _f, C.c_int, _f, _f, _f, C.POINTER(Push), _i32, _f]),
     "gca_fwd_hop2_up": (C.c_int, [_f, _f, _f, _i64, _f, _f, _f, C.c_int, _f, _f, _i64, _f, _i32, _i32, _f]),
+    "gca_fwd_hop2_up_add": (C.c_int, [_f, _f, _f, _i64, _f, _f, _f, C.c_int, _f, _f, _i64, _f, _i64, _f, _i32, _i32, _f]),
     "gca_bwd_scratch_bytes": (_sz, [_i32, _i32]),
     "gca_bwd_up": (C.c_int, [_f, _f, _i64, _f, _f, _f, _f, _f, C.POINTER(Push), _i32, _i32, _f]),
     "gca_bwd_up_project": (C.c_int, [_f, _f, _i64, _f, _f, _f, _f, C.POINTER(Push), _i32, _i32, _f]),
@@ -75,6 +76,8 @@ SIGNATURES = {
     "gca_bwd_finalize": (C.c_int, [_f, _f, _f, _f, C.c_int, _f, _f, _f, _f, _f, _i32, _i32, _f]),
     "gca_forward_workspace_bytes": (_sz, [_f, _i32, _i32]),
     "gca_forward": (C.c_int, [_f, _f, _i64, _f, _f, _f, _f, _f, C.c_int, C.c_int, _f, _f, _f, _f, _f, _i64, _i32, _i32, _f]),
+    "gca_forward_add": (C.c_int, [_f, _f, _i64, _f, _f, _f, _f, _f, C.c_int, C.c_int, _f, _f, _f, _f, _f, _i64, _f, _i64,
+                                  _i32, _i32, _f]),
     "gca_backward_workspace_bytes": (_sz, [_f, _i32, _i32]),
     "gca_backward": (C.c_int, [_f, _f, _i64, _f, _i64, _f, _f, _f, _f, _f, _f, _f, C.c_int, C.c_int, _f,
                                _f, _i64, _f, _f, _f, _f, _f, _i32, _i32, _f]),
@@ -88,6 +91,7 @@ SIGNATURES = {
     "gca_peer_close": (C.c_int, [_f]),
     "gca_layernorm_scratch_bytes": (_sz, [_i32]),
     "gca_layernorm_scale_fwd": (C.c_int, [_f, _i64, _f, _f, _f, C.c_float, _f, _i64, _f, _f, _i32, _i32, _f]),
+    "gca_layernorm_scale_add_fwd": (C.c_int, [_f, _i64, _f, _f, _f, C.c_float, _f, _i64, _f, _i64, _f, _f, _i32, _i32, _f]),
     "gca_layernorm_scale_bwd": (C.c_int, [_f, _i64, _f, _i64, _f, _f, _f, _f, _f, _f, _i64, _f, _f, _f, _f, _i32, _i32, _f]),
     "gca_nccl_available": (C.c_int, []),
     "gca_forward_nccl_workspace_bytes": (_sz, [_f, _i32, _i32, _i32]),

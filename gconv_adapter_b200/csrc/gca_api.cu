@@ -62,9 +62,11 @@ extern "C" int gca_fwd_hop1(const gca_graph* g, const float* Pp_full, const floa
                       nullptr, n, static_cast<cudaStream_t>(stream), 0, nullptr, push);
 }
 
-extern "C" int gca_fwd_hop2_up(const gca_graph* g, const float* Zp_full, const float* X, int64_t ldx, const float* Wu,
-                               const float* bu, const float* scalar, int skip, float* H2_local, float* Y, int64_t ldy,
-                               void* hub_scratch, int32_t d, int32_t r, gca_stream_t stream) {
+namespace {
+// gca_fwd_hop2_up (A = NULL) and gca_fwd_hop2_up_add (A = the addend, checked by the caller)
+int fwd_hop2_up(const gca_graph* g, const float* Zp_full, const float* X, int64_t ldx, const float* Wu, const float* bu,
+                const float* scalar, int skip, float* H2_local, const float* A, int64_t lda, float* Y, int64_t ldy,
+                void* hub_scratch, int32_t d, int32_t r, gca_stream_t stream) {
     if (!g || !Zp_full || !Wu || !bu || !H2_local || !Y || ldy < d) return GCA_ERR_INVALID_ARG;
     if (skip && (!X || ldx < d)) return GCA_ERR_INVALID_ARG;
     if (!shape_ok(d, r) || (ldy % 4) != 0 || (skip && (ldx % 4) != 0)) return GCA_ERR_UNSUPPORTED;
@@ -72,7 +74,23 @@ extern "C" int gca_fwd_hop2_up(const gca_graph* g, const float* Zp_full, const f
     const int n = g->row_end - g->row_begin;
     const PdlHint pdl_hint(n);
     return launch_hop_expand(r, true, csr_of(g, false, hub_scratch), Zp_full, Wu, bu, X, ldx, scalar, 1, skip ? 1 : 0, H2_local,
-                             Y, ldy, n, d, static_cast<cudaStream_t>(stream));
+                             Y, ldy, n, d, static_cast<cudaStream_t>(stream), A, lda);
+}
+inline bool addend_ok(const float* A, int64_t lda, int32_t d) { return A && lda >= d; }
+}  // namespace
+
+extern "C" int gca_fwd_hop2_up(const gca_graph* g, const float* Zp_full, const float* X, int64_t ldx, const float* Wu,
+                               const float* bu, const float* scalar, int skip, float* H2_local, float* Y, int64_t ldy,
+                               void* hub_scratch, int32_t d, int32_t r, gca_stream_t stream) {
+    return fwd_hop2_up(g, Zp_full, X, ldx, Wu, bu, scalar, skip, H2_local, nullptr, 0, Y, ldy, hub_scratch, d, r, stream);
+}
+
+extern "C" int gca_fwd_hop2_up_add(const gca_graph* g, const float* Zp_full, const float* X, int64_t ldx, const float* Wu,
+                                   const float* bu, const float* scalar, int skip, float* H2_local, const float* A, int64_t lda,
+                                   float* Y, int64_t ldy, void* hub_scratch, int32_t d, int32_t r, gca_stream_t stream) {
+    if (!addend_ok(A, lda, d)) return GCA_ERR_INVALID_ARG;
+    if ((lda % 4) != 0) return GCA_ERR_UNSUPPORTED;
+    return fwd_hop2_up(g, Zp_full, X, ldx, Wu, bu, scalar, skip, H2_local, A, lda, Y, ldy, hub_scratch, d, r, stream);
 }
 
 extern "C" size_t gca_bwd_scratch_bytes(int32_t d, int32_t r) {
@@ -196,10 +214,11 @@ extern "C" size_t gca_forward_workspace_bytes(const gca_graph* g, int32_t d, int
     return rw_bytes(g->row_end - g->row_begin, r) + hub_scratch_bytes(g);
 }
 
-extern "C" int gca_forward(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, const float* bd,
-                           const float* Wu, const float* bu, const float* scalar, int act, int skip, void* workspace,
-                           float* Zp_save, float* H1_save, float* H2_save, float* Y, int64_t ldy, int32_t d, int32_t r,
-                           gca_stream_t stream) {
+namespace {
+// gca_forward (A = NULL) and gca_forward_add: the same kernels and the same choice between them, A only changes the store
+int forward(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, const float* bd, const float* Wu, const float* bu,
+            const float* scalar, int act, int skip, void* workspace, float* Zp_save, float* H1_save, float* H2_save,
+            const float* A, int64_t lda, float* Y, int64_t ldy, int32_t d, int32_t r, gca_stream_t stream) {
     if (!g || !workspace) return GCA_ERR_INVALID_ARG;
     if (g->row_begin != 0 || g->row_end != g->N) return GCA_ERR_INVALID_ARG;   // partitioned graphs use the phases
     if ((reinterpret_cast<uintptr_t>(workspace) % kAlign) != 0) return GCA_ERR_WORKSPACE;
@@ -211,10 +230,28 @@ extern "C" int gca_forward(const gca_graph* g, const float* X, int64_t ldx, cons
     if (X && Wd && bd && Wu && bu && Zp_save && H2_save && Y && ldx >= d && ldy >= d && act >= GCA_ACT_NONE &&
         act <= GCA_ACT_SILU && (act != GCA_ACT_SILU || H1_save) && small_path_ok(g, d, r, static_cast<cudaStream_t>(stream)))
         return small_forward(g, X, ldx, Wd, bd, Wu, bu, scalar, act, skip, Pp, Zp_save, H1_save, H2_save, Y, ldy, d, r,
-                             static_cast<cudaStream_t>(stream));
+                             static_cast<cudaStream_t>(stream), A, lda);
     GCA_TRY(gca_fwd_project(g, X, ldx, Wd, Pp, nullptr, d, r, stream));
     GCA_TRY(gca_fwd_hop1(g, Pp, bd, act, Zp_save, H1_save, hub, nullptr, r, stream));
-    return gca_fwd_hop2_up(g, Zp_save, X, ldx, Wu, bu, scalar, skip, H2_save, Y, ldy, hub, d, r, stream);
+    return fwd_hop2_up(g, Zp_save, X, ldx, Wu, bu, scalar, skip, H2_save, A, lda, Y, ldy, hub, d, r, stream);
+}
+}  // namespace
+
+extern "C" int gca_forward(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, const float* bd,
+                           const float* Wu, const float* bu, const float* scalar, int act, int skip, void* workspace,
+                           float* Zp_save, float* H1_save, float* H2_save, float* Y, int64_t ldy, int32_t d, int32_t r,
+                           gca_stream_t stream) {
+    return forward(g, X, ldx, Wd, bd, Wu, bu, scalar, act, skip, workspace, Zp_save, H1_save, H2_save, nullptr, 0, Y, ldy, d, r,
+                   stream);
+}
+
+extern "C" int gca_forward_add(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, const float* bd,
+                               const float* Wu, const float* bu, const float* scalar, int act, int skip, void* workspace,
+                               float* Zp_save, float* H1_save, float* H2_save, const float* A, int64_t lda, float* Y, int64_t ldy,
+                               int32_t d, int32_t r, gca_stream_t stream) {
+    if (!addend_ok(A, lda, d)) return GCA_ERR_INVALID_ARG;
+    if ((lda % 4) != 0) return GCA_ERR_UNSUPPORTED;
+    return forward(g, X, ldx, Wd, bd, Wu, bu, scalar, act, skip, workspace, Zp_save, H1_save, H2_save, A, lda, Y, ldy, d, r, stream);
 }
 
 extern "C" size_t gca_backward_workspace_bytes(const gca_graph* g, int32_t d, int32_t r) {

@@ -134,6 +134,19 @@ __device__ __forceinline__ void stg4_stream(float* p, float4 v) {
     asm volatile("st.global.L1::no_allocate.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;"
                  :: "l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(l2_evict_first_policy()) : "memory");
 }
+// The addend A of the *_add entries (Y = ... + A).  Y == A is allowed, so A is read through the coherent path (not .nc,
+// whose data must stay unchanged for the kernel's lifetime), still without L1 allocation and L2 evict-first.
+__device__ __forceinline__ float4 ld4_addend(const float* p) {
+    float4 v;
+    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
+                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(l2_evict_first_policy()));
+    return v;
+}
+// y + a as one round-to-nearest add per element (never contracted into an FMA with the product that formed y), so the
+// fused sum has the bits of the separate `y + a`.
+__device__ __forceinline__ float4 f4_add_rn(float4 y, float4 a) {
+    return make_float4(__fadd_rn(y.x, a.x), __fadd_rn(y.y, a.y), __fadd_rn(y.z, a.z), __fadd_rn(y.w, a.w));
+}
 __device__ __forceinline__ float4 f4_add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
 __device__ __forceinline__ float4 f4_scale(float4 a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
 __device__ __forceinline__ float4 f4_shfl_xor(float4 v, int m) {

@@ -82,6 +82,10 @@ __device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void* src, uint
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
+// L2 prefetch of `bytes` (multiple of 16) bytes at a 16-byte aligned global address, no destination in the SM
+__device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {
+    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }

@@ -1,5 +1,6 @@
 // K3: hop + expansion.  r-wide gather-SpMM of a row tile fused with the [rows,R] x [R,d] expansion, bias, residual and
-// scalar (conv_up + skip + scalar ; gP -> gX):
+// scalar (conv_up + skip + scalar ; gP -> gX), and in the forward optionally + an addend A (ADD: parallel insertion,
+// Y = h + adapter(x) in the same pass; gca_fwd_hop2_up_add):
 //   k_hop_expand_tc    tcgen05 / TMEM accumulator, tensor-map TMA in and out, 128-row tiles  (r = 16 / 32, d % 64 == 0, d <= 256)
 //   k_hop_expand_mma   3xTF32 mma.sync, one kernel per 64-row tile                           (r = 16 / 32, other d)
 //   k_hop_expand       FFMA                                                                   (every other shape)
@@ -22,14 +23,14 @@ constexpr int kTileRows = 64;     // rows per CTA tile in k_hop_expand / k_hop_e
 // W is kept transposed in shared memory as WT[c][k] so a warp reads 512 contiguous bytes per c.
 // Warp w owns rows 8w..8w+7 of the tile, lane l the column quads l, l+32, ...
 // ------------------------------------------------------------------------------------------
-template <int R, bool W_IS_DR>
+template <int R, bool W_IS_DR, bool ADD>
 __global__ void __launch_bounds__(256, 2)
 k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, const float* __restrict__ dis,
              const float* __restrict__ F, const float* __restrict__ W, const float* __restrict__ bias,
              const float* __restrict__ resid, int64_t ldr, const float* __restrict__ scalar,
              int alpha_is_scalar, int use_resid, float* __restrict__ Hout, float* __restrict__ Out, int64_t ldo,
              int n, int d,
-    const int* __restrict__ hubitem, const float* __restrict__ hub_part) {
+    const int* __restrict__ hubitem, const float* __restrict__ hub_part, const float* addend, int64_t lda) {
     constexpr int LPG = R / 4, GPW = 32 / LPG;
     extern __shared__ __align__(16) float smem[];
     float* WT = smem;                 // [R][d]
@@ -94,6 +95,12 @@ k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
                     acc[i].z = fmaf(h.w, w3.z, acc[i].z); acc[i].w = fmaf(h.w, w3.w, acc[i].w);
                 }
             }
+            float4 xa[ADD ? 8 : 1];
+            if constexpr (ADD) {          // (issued after the expansion: the W and H operands are dead by now)
+#pragma unroll
+                for (int i = 0; i < 8; ++i)
+                    xa[i] = (r0 + i < n) ? ld4_addend(addend + (size_t)(r0 + i) * lda + q * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+            }
             float4 b4 = make_float4(0.f, 0.f, 0.f, 0.f);
             if (bias) b4 = ldg4(bias + q * 4);
 #pragma unroll
@@ -105,6 +112,7 @@ k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
                     y.x = fmaf(beta, xr[i].x, y.x); y.y = fmaf(beta, xr[i].y, y.y);
                     y.z = fmaf(beta, xr[i].z, y.z); y.w = fmaf(beta, xr[i].w, y.w);
                 }
+                if constexpr (ADD) y = f4_add_rn(y, xa[i]);
                 stg4_stream(Out + (size_t)(r0 + i) * ldo + q * 4, y);
             }
         }
@@ -119,14 +127,14 @@ k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
 // residual and writes the output as two float4 (columns cb+8t .. +7) for rows g and g+8 of every m-tile, i.e.
 // 8 rows x 128 contiguous bytes per warp instruction.
 // ------------------------------------------------------------------------------------------
-template <int R, bool W_IS_DR>
+template <int R, bool W_IS_DR, bool ADD>
 __global__ void __launch_bounds__(256, 2)
 k_hop_expand_mma(const int* __restrict__ rowptr, const int* __restrict__ colidx, const float* __restrict__ dis,
                  const float* __restrict__ F, const float* __restrict__ W, const float* __restrict__ bias,
                  const float* __restrict__ resid, int64_t ldr, const float* __restrict__ scalar,
                  int alpha_is_scalar, int use_resid, float* __restrict__ Hout, float* __restrict__ Out, int64_t ldo,
                  int n, int d,
-    const int* __restrict__ hubitem, const float* __restrict__ hub_part) {
+    const int* __restrict__ hubitem, const float* __restrict__ hub_part, const float* addend, int64_t lda) {
     constexpr int LPG = R / 4, GPW = 32 / LPG;
     constexpr int RS = R + 4;                       // padded row stride of the H tile
     constexpr int KS = R / 8;                       // k-steps
@@ -196,7 +204,7 @@ k_hop_expand_mma(const int* __restrict__ rowptr, const int* __restrict__ colidx,
             const bool o0 = oc < d, o1 = oc1 < d;
             float4 b4a = make_float4(0.f, 0.f, 0.f, 0.f), b4b = b4a;
             if (bias) { if (o0) b4a = ldg4(bias + oc); if (o1) b4b = ldg4(bias + oc1); }
-#pragma unroll 2
+#pragma unroll(ADD ? 1 : 2)                                 // (ADD: the addend's registers do not fit twice)
             for (int mt = 0; mt < kTileRows / 16; ++mt) {
                 const int r0 = trow + mt * 16 + g, r1 = r0 + 8;
                 float4 x0a, x0b, x1a, x1b;
@@ -231,13 +239,28 @@ k_hop_expand_mma(const int* __restrict__ rowptr, const int* __restrict__ colidx,
                     }
                     return y;
                 };
-                if (r0 < n) {
-                    if (o0) stg4_stream(Out + (size_t)r0 * ldo + oc, fin(acc[0][0], acc[1][0], acc[2][0], acc[3][0], b4a, x0a));
-                    if (o1) stg4_stream(Out + (size_t)r0 * ldo + oc1, fin(acc[0][1], acc[1][1], acc[2][1], acc[3][1], b4b, x0b));
-                }
-                if (r1 < n) {
-                    if (o0) stg4_stream(Out + (size_t)r1 * ldo + oc, fin(acc[0][2], acc[1][2], acc[2][2], acc[3][2], b4a, x1a));
-                    if (o1) stg4_stream(Out + (size_t)r1 * ldo + oc1, fin(acc[0][3], acc[1][3], acc[2][3], acc[3][3], b4b, x1b));
+                if constexpr (!ADD) {
+                    if (r0 < n) {
+                        if (o0) stg4_stream(Out + (size_t)r0 * ldo + oc, fin(acc[0][0], acc[1][0], acc[2][0], acc[3][0], b4a, x0a));
+                        if (o1) stg4_stream(Out + (size_t)r0 * ldo + oc1, fin(acc[0][1], acc[1][1], acc[2][1], acc[3][1], b4b, x0b));
+                    }
+                    if (r1 < n) {
+                        if (o0) stg4_stream(Out + (size_t)r1 * ldo + oc, fin(acc[0][2], acc[1][2], acc[2][2], acc[3][2], b4a, x1a));
+                        if (o1) stg4_stream(Out + (size_t)r1 * ldo + oc1, fin(acc[0][3], acc[1][3], acc[2][3], acc[3][3], b4b, x1b));
+                    }
+                } else {
+                    float4 a0a, a0b, a1a, a1b;
+                    a0a = a0b = a1a = a1b = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (r0 < n) { if (o0) a0a = ld4_addend(addend + (size_t)r0 * lda + oc); if (o1) a0b = ld4_addend(addend + (size_t)r0 * lda + oc1); }
+                    if (r1 < n) { if (o0) a1a = ld4_addend(addend + (size_t)r1 * lda + oc); if (o1) a1b = ld4_addend(addend + (size_t)r1 * lda + oc1); }
+                    if (r0 < n) {
+                        if (o0) stg4_stream(Out + (size_t)r0 * ldo + oc, f4_add_rn(fin(acc[0][0], acc[1][0], acc[2][0], acc[3][0], b4a, x0a), a0a));
+                        if (o1) stg4_stream(Out + (size_t)r0 * ldo + oc1, f4_add_rn(fin(acc[0][1], acc[1][1], acc[2][1], acc[3][1], b4b, x0b), a0b));
+                    }
+                    if (r1 < n) {
+                        if (o0) stg4_stream(Out + (size_t)r1 * ldo + oc, f4_add_rn(fin(acc[0][2], acc[1][2], acc[2][2], acc[3][2], b4a, x1a), a1a));
+                        if (o1) stg4_stream(Out + (size_t)r1 * ldo + oc1, f4_add_rn(fin(acc[0][3], acc[1][3], acc[2][3], acc[3][3], b4b, x1b), a1b));
+                    }
                 }
             }
         }
@@ -273,14 +296,15 @@ constexpr size_t hop_expand_tc_smem(int d) {
     return (size_t)2 * R * d * 4 + (size_t)4 * R * kTcRows * 4 + (size_t)4 * tc_slots<R>() * kTcSlotBytes + (size_t)d * 4 + 64 * 8 + 64 + 1024;
 }
 
-template <int R, bool W_IS_DR>
+template <int R, bool W_IS_DR, bool ADD>
 __global__ void __launch_bounds__(512, 1)
 k_hop_expand_tc(const int* __restrict__ rowptr, const int* __restrict__ colidx, const float* __restrict__ dis,
                 const float* __restrict__ F, const float* __restrict__ W, const float* __restrict__ bias,
                 const float* __restrict__ resid, int64_t ldr, const float* __restrict__ scalar,
                 int alpha_is_scalar, int use_resid, float* __restrict__ Hout, float* __restrict__ Out, int64_t ldo,
                 int n, int d, const int* __restrict__ hubitem, const float* __restrict__ hub_part,
-                const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_y, int pregathered) {
+                const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_y, int pregathered,
+                const float* addend, int64_t lda) {
     constexpr int LPG = R / 4, GPW = 32 / LPG;
     constexpr int kTcSlots = tc_slots<R>();
     constexpr int SCA = (kTcRows >> 3) * 128;          // bytes between 4-column K chunks of the H tile
@@ -521,6 +545,14 @@ k_hop_expand_tc(const int* __restrict__ rowptr, const int* __restrict__ colidx, 
         if (use_resid && lane == 0 && tk >= 0)
             for (int c_ = 0; c_ < lead; ++c_) issue_load(tk, c_, c_);
         const int sw = lane & 7;                                   // 16-byte chunk j of row `lane` sits at chunk j ^ (lane % 8)
+        // ADD: the addend's 32 columns from col0 of row `lane` of `tile` (zeros past the last row)
+        auto load_half = [&](int tile, int col0, float4 (&dst)[8]) {
+            const int row = tile * kTcRows + q * 32 + lane;
+            const bool ok = row < n;
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                dst[j] = ok ? ld4_addend(addend + (size_t)row * lda + col0 + 4 * j) : make_float4(0.f, 0.f, 0.f, 0.f);
+        };
         int it = 0;
         for (int k = 0; tk >= 0; ++k) {
             const int b = k & 1;
@@ -530,43 +562,97 @@ k_hop_expand_tc(const int* __restrict__ rowptr, const int* __restrict__ colidx, 
             const uint32_t tb = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * 256);
             for (int c = 0; c < nchunk; ++c, ++it) {
                 const int slot = it % kTcSlots;
-                float acc[kTcChunk];
-                tmem_ld32(tb + (uint32_t)(c * kTcChunk), acc);
-                tmem_ld32(tb + (uint32_t)(c * kTcChunk + 32), acc + 32);
-                if (use_resid) mbar_wait(xfull(q, slot), (uint32_t)((it / kTcSlots) & 1));
-                tmem_ld_wait();
-                if (c == nchunk - 1) {                              // accumulator stage can be overwritten
-                    tc::tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) tc::mbar_arrive(tempty(b));
-                }
-                uint8_t* slotp = myslots + (size_t)slot * kTcSlotBytes + (size_t)lane * 128;
-                const float4* bs = reinterpret_cast<const float4*>(bias_s + c * kTcChunk);
-                // all loads of a half chunk first, then the arithmetic, then the stores: the compiler cannot tell that
-                // the swizzled in-place stores do not alias the later loads and would otherwise serialise them
+                if constexpr (!ADD) {
+                    float acc[kTcChunk];
+                    tmem_ld32(tb + (uint32_t)(c * kTcChunk), acc);
+                    tmem_ld32(tb + (uint32_t)(c * kTcChunk + 32), acc + 32);
+                    if (use_resid) mbar_wait(xfull(q, slot), (uint32_t)((it / kTcSlots) & 1));
+                    tmem_ld_wait();
+                    if (c == nchunk - 1) {                              // accumulator stage can be overwritten
+                        tc::tc_fence_before();
+                        __syncwarp();
+                        if (lane == 0) tc::mbar_arrive(tempty(b));
+                    }
+                    uint8_t* slotp = myslots + (size_t)slot * kTcSlotBytes + (size_t)lane * 128;
+                    const float4* bs = reinterpret_cast<const float4*>(bias_s + c * kTcChunk);
+                    // all loads of a half chunk first, then the arithmetic, then the stores: the compiler cannot tell that
+                    // the swizzled in-place stores do not alias the later loads and would otherwise serialise them
 #pragma unroll
-                for (int h = 0; h < 4; ++h) {                       // quarter chunks of 16 columns
-                    float4 xv[4], bv[4];
+                    for (int h = 0; h < 4; ++h) {                       // quarter chunks of 16 columns
+                        float4 xv[4], bv[4];
 #pragma unroll
-                    for (int jj = 0; jj < 4; ++jj) {
-                        const int j = h * 4 + jj;
-                        bv[jj] = bs[j];
-                        xv[jj] = use_resid ? *reinterpret_cast<const float4*>(slotp + (j >> 3) * kTcBoxBytes + (((j & 7) ^ sw) << 4))
-                                           : make_float4(0.f, 0.f, 0.f, 0.f);
+                        for (int jj = 0; jj < 4; ++jj) {
+                            const int j = h * 4 + jj;
+                            bv[jj] = bs[j];
+                            xv[jj] = use_resid ? *reinterpret_cast<const float4*>(slotp + (j >> 3) * kTcBoxBytes + (((j & 7) ^ sw) << 4))
+                                               : make_float4(0.f, 0.f, 0.f, 0.f);
+                        }
+#pragma unroll
+                        for (int jj = 0; jj < 4; ++jj) {
+                            const int j = h * 4 + jj;
+                            float4 y = make_float4(alpha * (acc[4 * j] + bv[jj].x), alpha * (acc[4 * j + 1] + bv[jj].y),
+                                                   alpha * (acc[4 * j + 2] + bv[jj].z), alpha * (acc[4 * j + 3] + bv[jj].w));
+                            y.x = fmaf(beta, xv[jj].x, y.x); y.y = fmaf(beta, xv[jj].y, y.y);
+                            y.z = fmaf(beta, xv[jj].z, y.z); y.w = fmaf(beta, xv[jj].w, y.w);
+                            xv[jj] = y;
+                        }
+#pragma unroll
+                        for (int jj = 0; jj < 4; ++jj) {
+                            const int j = h * 4 + jj;
+                            *reinterpret_cast<float4*>(slotp + (j >> 3) * kTcBoxBytes + (((j & 7) ^ sw) << 4)) = xv[jj];
+                        }
+                    }
+                } else {
+                    // Y = (...) + A.  Lane = row; A comes in 32-column halves of 128-bit loads into registers (the 128
+                    // registers of the kernel leave no room for a whole chunk, or for the next half, next to the
+                    // accumulator), issued before the half waits on TMEM and the residual.  The next chunk's bytes are
+                    // prefetched into L2 one chunk ahead (no shared memory is left for a ring of A), so those loads hit L2.
+                    // Every load of chunk c is consumed before chunk c's store is issued, which is what makes Y == A safe.
+                    uint8_t* slotp = myslots + (size_t)slot * kTcSlotBytes + (size_t)lane * 128;
+                    const float4* bs = reinterpret_cast<const float4*>(bias_s + c * kTcChunk);
+                    {
+                        const int cn = c + 1 < nchunk ? c + 1 : 0, tile_n = c + 1 < nchunk ? tk : tk1;
+                        const int prow = tile_n * kTcRows + q * 32 + lane;
+                        if (tile_n >= 0 && prow < n) prefetch_l2_bulk(addend + (size_t)prow * lda + cn * kTcChunk, kTcChunk * 4);
                     }
 #pragma unroll
-                    for (int jj = 0; jj < 4; ++jj) {
-                        const int j = h * 4 + jj;
-                        float4 y = make_float4(alpha * (acc[4 * j] + bv[jj].x), alpha * (acc[4 * j + 1] + bv[jj].y),
-                                               alpha * (acc[4 * j + 2] + bv[jj].z), alpha * (acc[4 * j + 3] + bv[jj].w));
-                        y.x = fmaf(beta, xv[jj].x, y.x); y.y = fmaf(beta, xv[jj].y, y.y);
-                        y.z = fmaf(beta, xv[jj].z, y.z); y.w = fmaf(beta, xv[jj].w, y.w);
-                        xv[jj] = y;
-                    }
+                    for (int hh = 0; hh < 2; ++hh) {
+                        float4 cur[8];
+                        load_half(tk, c * kTcChunk + hh * 32, cur);
+                        float acc[32];
+                        tmem_ld32(tb + (uint32_t)(c * kTcChunk + hh * 32), acc);
+                        if (hh == 0 && use_resid) mbar_wait(xfull(q, slot), (uint32_t)((it / kTcSlots) & 1));
+                        tmem_ld_wait();
+                        if (hh == 1 && c == nchunk - 1) {                   // accumulator stage can be overwritten
+                            tc::tc_fence_before();
+                            __syncwarp();
+                            if (lane == 0) tc::mbar_arrive(tempty(b));
+                        }
 #pragma unroll
-                    for (int jj = 0; jj < 4; ++jj) {
-                        const int j = h * 4 + jj;
-                        *reinterpret_cast<float4*>(slotp + (j >> 3) * kTcBoxBytes + (((j & 7) ^ sw) << 4)) = xv[jj];
+                        for (int h2 = 0; h2 < 4; ++h2) {                   // batches of 2 float4 (registers are at the cap)
+                            float4 xv[2], bv[2];
+#pragma unroll
+                            for (int jj = 0; jj < 2; ++jj) {
+                                const int j = hh * 8 + h2 * 2 + jj;
+                                bv[jj] = bs[j];
+                                xv[jj] = use_resid ? *reinterpret_cast<const float4*>(slotp + (j >> 3) * kTcBoxBytes + (((j & 7) ^ sw) << 4))
+                                                   : make_float4(0.f, 0.f, 0.f, 0.f);
+                            }
+#pragma unroll
+                            for (int jj = 0; jj < 2; ++jj) {
+                                const int e = h2 * 2 + jj;
+                                float4 y = make_float4(alpha * (acc[4 * e] + bv[jj].x), alpha * (acc[4 * e + 1] + bv[jj].y),
+                                                       alpha * (acc[4 * e + 2] + bv[jj].z), alpha * (acc[4 * e + 3] + bv[jj].w));
+                                y.x = fmaf(beta, xv[jj].x, y.x); y.y = fmaf(beta, xv[jj].y, y.y);
+                                y.z = fmaf(beta, xv[jj].z, y.z); y.w = fmaf(beta, xv[jj].w, y.w);
+                                xv[jj] = f4_add_rn(y, cur[e]);
+                            }
+#pragma unroll
+                            for (int jj = 0; jj < 2; ++jj) {
+                                const int j = hh * 8 + h2 * 2 + jj;
+                                *reinterpret_cast<float4*>(slotp + (j >> 3) * kTcBoxBytes + (((j & 7) ^ sw) << 4)) = xv[jj];
+                            }
+                        }
                     }
                 }
                 tc::fence_proxy_async();                           // generic-proxy writes -> visible to the bulk store
@@ -599,10 +685,11 @@ k_hop_expand_tc(const int* __restrict__ rowptr, const int* __restrict__ colidx, 
     }
 }
 
-template <int R, bool W_IS_DR>
+template <int R, bool W_IS_DR, bool ADD>
 int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
                         const float* bias, const float* resid, int64_t ldr, const float* scalar, int alpha_is_scalar,
-                        int use_resid, float* Hout, float* Out, int64_t ldo, int n, int d, cudaStream_t st) {
+                        int use_resid, float* Hout, float* Out, int64_t ldo, int n, int d, const float* addend, int64_t lda,
+                        cudaStream_t st) {
     if (n == 0) return GCA_OK;
     GCA_TRY(launch_hub_partials(R, c, F, st));
     const int* rowptr = c.rowptr; const int* colidx = c.colidx; const float* dis = c.dis;
@@ -625,28 +712,29 @@ int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
                                        W_IS_DR ? "hop_plain_fwd" : "hop_plain_bwd"));
                 const char* prof_k3 = pregathered ? (W_IS_DR ? "expand_fwd" : "expand_bwd") : (W_IS_DR ? "hop_expand_fwd" : "hop_expand_bwd");
                 const size_t smem_tc = hop_expand_tc_smem<R>(d);
-                GCA_TRY(set_smem(k_hop_expand_tc<R, W_IS_DR>, smem_tc));
+                GCA_TRY(set_smem(k_hop_expand_tc<R, W_IS_DR, ADD>, smem_tc));
                 const int ntiles_t = (n + kTcRows - 1) / kTcRows;
                 const int grid_t = ntiles_t < num_sms() ? ntiles_t : num_sms();
                 {
                     ProfScope ps(prof_k3, st, "tcgen05");
-                    GCA_CUDA(launch_pdl(k_hop_expand_tc<R, W_IS_DR>, dim3(grid_t), dim3(512), smem_tc, st, rowptr, colidx, dis, F, W, bias,
-                                        resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, c.hubitem, c.hub_part, tm_x, tm_y,
-                                        pregathered));
+                    GCA_CUDA(launch_pdl(k_hop_expand_tc<R, W_IS_DR, ADD>, dim3(grid_t), dim3(512), smem_tc, st, rowptr, colidx, dis, F, W,
+                                        bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, c.hubitem, c.hub_part,
+                                        tm_x, tm_y, pregathered, addend, lda));
                 }
                 GCA_LAUNCH_OK();
                 return GCA_OK;
             }
             const size_t smem_m = sizeof(uint32_t) * ((size_t)2 * R * (d + 1) + (size_t)2 * kTileRows * (R + 4));
             if (smem_m <= 200 * 1024) {
-                GCA_TRY(set_smem(k_hop_expand_mma<R, W_IS_DR>, smem_m));
+                GCA_TRY(set_smem(k_hop_expand_mma<R, W_IS_DR, ADD>, smem_m));
                 const int ntiles_m = (n + kTileRows - 1) / kTileRows;
                 const int per_sm = smem_m <= 100 * 1024 ? 2 : 1;
                 const int grid_m = ntiles_m < per_sm * num_sms() ? ntiles_m : per_sm * num_sms();
                 {
                     ProfScope ps(W_IS_DR ? "hop_expand_fwd" : "hop_expand_bwd", st, "mma");
-                    k_hop_expand_mma<R, W_IS_DR><<<grid_m, 256, smem_m, st>>>(rowptr, colidx, dis, F, W, bias, resid, ldr, scalar,
-                                                                              alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, c.hubitem, c.hub_part);
+                    k_hop_expand_mma<R, W_IS_DR, ADD><<<grid_m, 256, smem_m, st>>>(rowptr, colidx, dis, F, W, bias, resid, ldr, scalar,
+                                                                                   alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, c.hubitem,
+                                                                                   c.hub_part, addend, lda);
                 }
                 GCA_LAUNCH_OK();
                 return GCA_OK;
@@ -655,13 +743,14 @@ int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
     }
     const size_t smem = sizeof(float) * ((size_t)R * d + (size_t)kTileRows * R);
     if (smem > 200 * 1024) return GCA_ERR_UNSUPPORTED;
-    GCA_TRY(set_smem(k_hop_expand<R, W_IS_DR>, smem));
+    GCA_TRY(set_smem(k_hop_expand<R, W_IS_DR, ADD>, smem));
     const int ntiles = (n + kTileRows - 1) / kTileRows;
     const int grid = ntiles < 2 * num_sms() ? ntiles : 2 * num_sms();
     {
         ProfScope ps(W_IS_DR ? "hop_expand_fwd" : "hop_expand_bwd", st, "ffma");
-        k_hop_expand<R, W_IS_DR><<<grid, 256, smem, st>>>(rowptr, colidx, dis, F, W, bias, resid, ldr, scalar,
-                                                           alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, c.hubitem, c.hub_part);
+        k_hop_expand<R, W_IS_DR, ADD><<<grid, 256, smem, st>>>(rowptr, colidx, dis, F, W, bias, resid, ldr, scalar,
+                                                                alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, c.hubitem, c.hub_part,
+                                                                addend, lda);
     }
     GCA_LAUNCH_OK();
     return GCA_OK;
@@ -671,11 +760,19 @@ int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
 
 int launch_hop_expand(int r, bool w_is_dr, const Csr& c, const float* F, const float* W, const float* bias, const float* resid,
                       int64_t ldr, const float* scalar, int alpha_is_scalar, int use_resid, float* Hout, float* Out, int64_t ldo,
-                      int n, int d, cudaStream_t st) {
-    if (w_is_dr) {
-        GCA_DISPATCH_R(r, (launch_hop_expand_t<R_, true>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, st)));
+                      int n, int d, cudaStream_t st, const float* addend, int64_t lda) {
+    // the addend is forward-only (Y = ... + A); the variant choice inside does not depend on it
+    if (w_is_dr && addend) {
+        GCA_DISPATCH_R(r, (launch_hop_expand_t<R_, true, true>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo,
+                                                               n, d, addend, lda, st)));
     }
-    GCA_DISPATCH_R(r, (launch_hop_expand_t<R_, false>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo, n, d, st)));
+    if (addend) return GCA_ERR_UNSUPPORTED;
+    if (w_is_dr) {
+        GCA_DISPATCH_R(r, (launch_hop_expand_t<R_, true, false>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out,
+                                                                ldo, n, d, nullptr, 0, st)));
+    }
+    GCA_DISPATCH_R(r, (launch_hop_expand_t<R_, false, false>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo,
+                                                             n, d, nullptr, 0, st)));
 }
 
 }  // namespace gca

@@ -98,10 +98,11 @@ int launch_hop(int r, bool bwd, const Csr& c, const float* F, const float* bias,
                const gca_push* push = nullptr);
 // copy a finished local shard to the peers (producers without a fused push)
 int launch_push_rows(const float* src, size_t nfloats, const gca_push* push, cudaStream_t st);
-// K3: hop + expansion  Out = alpha (H W + bias) + beta Resid   (w_is_dr: W stored [d, r], else [r, d])
+// K3: hop + expansion  Out = alpha (H W + bias) + beta Resid [+ addend]   (w_is_dr: W stored [d, r], else [r, d]).
+// addend (w_is_dr only): added to every output element with one round-to-nearest add; may equal Out with lda == ldo.
 int launch_hop_expand(int r, bool w_is_dr, const Csr& c, const float* F, const float* W, const float* bias, const float* resid,
                       int64_t ldr, const float* scalar, int alpha_is_scalar, int use_resid, float* Hout, float* Out, int64_t ldo,
-                      int n, int d, cudaStream_t st);
+                      int n, int d, cudaStream_t st, const float* addend = nullptr, int64_t lda = 0);
 // K4: per-CTA partials of G[r, d] = H^T A (+ column sums of A, <A, B>)
 int launch_wgrad(int r, const float* A, int64_t lda, const float* H, const float* B, int64_t ldb, float* partG, float* partCol,
                  float* partDot, int* header, int slot, int n, int d, cudaStream_t st);
@@ -124,7 +125,7 @@ int launch_dense_stream(int r, const DenseStreamArgs& a, cudaStream_t st);
 bool small_path_ok(const gca_graph* g, int d, int r, cudaStream_t st);
 int small_forward(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, const float* bd, const float* Wu,
                   const float* bu, const float* scalar, int act, int skip, float* P, float* Zp, float* H1, float* H2, float* Y,
-                  int64_t ldy, int d, int r, cudaStream_t st);
+                  int64_t ldy, int d, int r, cudaStream_t st, const float* A = nullptr, int64_t lda = 0);
 int small_backward(const gca_graph* g, const float* gY, int64_t ldg, const float* X, int64_t ldx, const float* Zp,
                    const float* H1, const float* H2, const float* Wd, const float* Wu, const float* bu, const float* scalar,
                    int act, int skip, float* gH2, float* gH1, float* gP, float* gX, int64_t ldgx, const Scratch& S, float* gWd,

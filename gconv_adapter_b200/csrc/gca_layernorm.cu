@@ -25,11 +25,11 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
-template <int VPL>   // float4s per lane: d <= 128 * VPL
+template <int VPL, bool ADD>   // float4s per lane: d <= 128 * VPL ; ADD: Y = ... + A (gca_layernorm_scale_add_fwd)
 __global__ void __launch_bounds__(kLnThreads)
 k_ln_fwd(const float* __restrict__ X, int64_t ldx, const float* __restrict__ gamma, const float* __restrict__ beta,
          const float* __restrict__ scalar, float eps, float* __restrict__ Y, int64_t ldy, float* __restrict__ mean_out,
-         float* __restrict__ rstd_out, int n, int d) {
+         float* __restrict__ rstd_out, int n, int d, const float* A, int64_t lda) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int nq = d >> 2;
     const float s = scalar ? __ldg(scalar) : 1.f;
@@ -52,6 +52,14 @@ k_ln_fwd(const float* __restrict__ X, int64_t ldx, const float* __restrict__ gam
             x[v] = q < nq ? ldg4_stream(X + (size_t)row * ldx + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
             sum += (x[v].x + x[v].y) + (x[v].z + x[v].w);
         }
+        float4 av[ADD ? VPL : 1];
+        if constexpr (ADD) {
+#pragma unroll
+            for (int v = 0; v < VPL; ++v) {
+                const int q = lane + 32 * v;
+                av[v] = q < nq ? ld4_addend(A + (size_t)row * lda + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        }
         const float mean = warp_sum(sum) * inv_d;
         float sq = 0.f;
 #pragma unroll
@@ -72,6 +80,7 @@ k_ln_fwd(const float* __restrict__ X, int64_t ldx, const float* __restrict__ gam
                 y.y = s * fmaf((x[v].y - mean) * rstd, gm[v].y, bt[v].y);
                 y.z = s * fmaf((x[v].z - mean) * rstd, gm[v].z, bt[v].z);
                 y.w = s * fmaf((x[v].w - mean) * rstd, gm[v].w, bt[v].w);
+                if constexpr (ADD) y = f4_add_rn(y, av[v]);
                 stg4_stream(Y + (size_t)row * ldy + 4 * q, y);
             }
         }
@@ -199,14 +208,15 @@ k_ln_bwd_finalize(const float* __restrict__ partG, const float* __restrict__ par
 
 inline size_t ln_scratch_bytes(int d) { return align_up(sizeof(float) * ((size_t)kLnMaxParts * 2 * d + kLnMaxParts)); }
 
-template <int VPL>
+template <int VPL, bool ADD>
 int ln_fwd_t(const float* X, int64_t ldx, const float* gamma, const float* beta, const float* scalar, float eps, float* Y,
-             int64_t ldy, float* mean, float* rstd, int n, int d, cudaStream_t st) {
+             int64_t ldy, float* mean, float* rstd, int n, int d, const float* A, int64_t lda, cudaStream_t st) {
     int grid = (n + kLnWarps - 1) / kLnWarps;
     if (grid > 8 * num_sms()) grid = 8 * num_sms();
     {
         ProfScope ps("layernorm_fwd", st);
-        GCA_CUDA(launch_pdl(k_ln_fwd<VPL>, dim3(grid), dim3(kLnThreads), 0, st, X, ldx, gamma, beta, scalar, eps, Y, ldy, mean, rstd, n, d));
+        GCA_CUDA(launch_pdl(k_ln_fwd<VPL, ADD>, dim3(grid), dim3(kLnThreads), 0, st, X, ldx, gamma, beta, scalar, eps, Y, ldy, mean, rstd,
+                            n, d, A, lda));
     }
     GCA_LAUNCH_OK();
     return GCA_OK;
@@ -267,7 +277,19 @@ extern "C" int gca_layernorm_scale_fwd(const float* X, int64_t ldx, const float*
     if (n == 0) return GCA_OK;
     const PdlHint pdl_hint(n);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    GCA_DISPATCH_VPL(d, (ln_fwd_t<V_>(X, ldx, gamma, beta, scalar, eps, Y, ldy, mean, rstd, n, d, st)));
+    GCA_DISPATCH_VPL(d, (ln_fwd_t<V_, false>(X, ldx, gamma, beta, scalar, eps, Y, ldy, mean, rstd, n, d, nullptr, 0, st)));
+}
+
+extern "C" int gca_layernorm_scale_add_fwd(const float* X, int64_t ldx, const float* gamma, const float* beta,
+                                           const float* scalar, float eps, const float* A, int64_t lda, float* Y, int64_t ldy,
+                                           float* mean, float* rstd, int32_t n, int32_t d, gca_stream_t stream) {
+    if (!mean || !rstd || !(eps >= 0.f)) return GCA_ERR_INVALID_ARG;
+    if (!X || !A || !Y || n < 0 || d <= 0) return GCA_ERR_INVALID_ARG;
+    if (!ln_args_ok(X, Y, ldx, ldy, n, d) || !ln_args_ok(A, Y, lda, ldy, n, d)) return GCA_ERR_UNSUPPORTED;
+    if (n == 0) return GCA_OK;
+    const PdlHint pdl_hint(n);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    GCA_DISPATCH_VPL(d, (ln_fwd_t<V_, true>(X, ldx, gamma, beta, scalar, eps, Y, ldy, mean, rstd, n, d, A, lda, st)));
 }
 
 extern "C" int gca_layernorm_scale_bwd(const float* gY, int64_t ldg, const float* X, int64_t ldx, const float* gamma,

@@ -6,7 +6,7 @@
 //
 //   forward   A  P'  = dis * (X Wd^T)                     warp per row, reduce-scatter over the lanes
 //             B  Z'  = dis * act(dis * (A' P') + bd)      lane group (r/4 lanes) per row
-//             C  H2  = dis * (A' Z') ;  Y = s (H2 Wu^T + bu [+ X])
+//             C  H2  = dis * (A' Z') ;  Y = s (H2 Wu^T + bu [+ X]) [+ A]   (A: gca_forward_add's addend)
 //   backward  A  gH2' = dis * s * (gY Wu)  ;  per-CTA partials of gY^T H2 and of the column sums of gY
 //             B  gH1' = dis * act'(.) * dis * (A'^T gH2') ; per-CTA partials of gbd
 //             C  gP  = dis * (A'^T gH1') ;  gX = gP Wd [+ s gY]
@@ -45,6 +45,7 @@ struct SmallFwd {
     int act, skip;
     float* P; float* Zp; float* H1; float* H2; float* Y; int64_t ldy;
     int n, d;
+    const float* A; int64_t lda;      // addend of gca_forward_add (k_small_fwd<R, true> only)
 };
 
 struct SmallBwd {
@@ -220,7 +221,7 @@ __device__ __forceinline__ float block_sum_ordered(float v, float* s_red) {     
     return s_red[0];
 }
 
-template <int R>
+template <int R, bool ADD>
 __global__ void __launch_bounds__(kSmallThreads) k_small_fwd(const SmallFwd a) {
     extern __shared__ float sm[];
     constexpr int LPG = R / 4, GPW = 32 / LPG;
@@ -281,7 +282,8 @@ __global__ void __launch_bounds__(kSmallThreads) k_small_fwd(const SmallFwd a) {
 #pragma unroll
                 for (int j = 0; j < R; ++j) y = fmaf(h[j], Wut_s[j * d + c], y);
                 if (a.skip) y += __ldg(xr + c);
-                yr[c] = s * y;
+                if constexpr (ADD) yr[c] = __fadd_rn(s * y, __ldcg(a.A + (size_t)rg * a.lda + c));   // (coherent: Y may be A)
+                else yr[c] = s * y;
             }
         }
     }
@@ -480,13 +482,13 @@ inline int small_grid(int n, int limit) {
     return grid < 1 ? 1 : grid;
 }
 
-template <int R>
+template <int R, bool ADD>
 int small_forward_t(const SmallFwd& a, cudaStream_t st) {
     const size_t smem = sizeof(float) * 2 * R * a.d;
-    GCA_TRY(set_smem(k_small_fwd<R>, smem));
-    const int limit = coop_grid_limit(k_small_fwd<R>, smem);
+    GCA_TRY(set_smem(k_small_fwd<R, ADD>, smem));
+    const int limit = coop_grid_limit(k_small_fwd<R, ADD>, smem);
     if (limit < 1) return GCA_ERR_UNSUPPORTED;
-    return launch_coop(k_small_fwd<R>, a, small_grid(a.n, limit), smem, st, "small_fwd");
+    return launch_coop(k_small_fwd<R, ADD>, a, small_grid(a.n, limit), smem, st, "small_fwd");
 }
 
 template <int R>
@@ -517,9 +519,10 @@ bool small_path_ok(const gca_graph* g, int d, int r, cudaStream_t st) {
 
 int small_forward(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, const float* bd, const float* Wu,
                   const float* bu, const float* scalar, int act, int skip, float* P, float* Zp, float* H1, float* H2, float* Y,
-                  int64_t ldy, int d, int r, cudaStream_t st) {
-    SmallFwd a{g->rowptr, g->colidx, g->dis, X, ldx, Wd, bd, Wu, bu, scalar, act, skip, P, Zp, H1, H2, Y, ldy, g->N, d};
-    GCA_DISPATCH_R(r, (small_forward_t<R_>(a, st)));
+                  int64_t ldy, int d, int r, cudaStream_t st, const float* A, int64_t lda) {
+    SmallFwd a{g->rowptr, g->colidx, g->dis, X, ldx, Wd, bd, Wu, bu, scalar, act, skip, P, Zp, H1, H2, Y, ldy, g->N, d, A, lda};
+    if (A) { GCA_DISPATCH_R(r, (small_forward_t<R_, true>(a, st))); }
+    GCA_DISPATCH_R(r, (small_forward_t<R_, false>(a, st)));
 }
 
 int small_backward(const gca_graph* g, const float* gY, int64_t ldg, const float* X, int64_t ldx, const float* Zp,

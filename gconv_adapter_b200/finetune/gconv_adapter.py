@@ -7,7 +7,8 @@ defaults (:23-26), same ``ValueError`` messages (:37,51,61), same parameter name
 (:73-78, drawing from the torch RNG in the order PyG's constructors + the reference do), same
 call signature ``forward(x, edge_index, edge_attr=None)`` (:80) with ``edge_attr`` ignored, x of
 shape ``[N, d]`` or ``[1, N, d]``, and the same op order skip -> normalization -> scalar
-(:94-106).  The arithmetic runs as hand-written CUDA (include/gca.h); there is NO CPU path:
+(:94-106).  ``forward(..., add_to=h)`` returns ``h + forward(...)`` (the reference's parallel insertion), with the
+add done in the store of the last kernel where the operands allow.  The arithmetic runs as hand-written CUDA (include/gca.h); there is NO CPU path:
 a CPU tensor, or a missing libgca.so, raises ``RuntimeError``.
 """
 from __future__ import annotations
@@ -92,7 +93,8 @@ class _GConvAdapterFunction(torch.autograd.Function):
     direction, carved into the tensors the kernels need, and one C call."""
 
     @staticmethod
-    def forward(ctx, x, w_down, b_down, w_up, b_up, scalar, graph: GraphStructure, act: int, skip: bool):
+    def forward(ctx, x, w_down, b_down, w_up, b_up, scalar, graph: GraphStructure, act: int, skip: bool, addend=None):
+        """``addend`` (optional, [n, d] fp32): Y += addend inside the last kernel (gca_forward_add); its gradient is gY."""
         lib = _cabi.load()
         x, ldx = kernel_operand(x)
         n, d = x.shape
@@ -114,9 +116,17 @@ class _GConvAdapterFunction(torch.autograd.Function):
         zp_ptr, h2_ptr = base, base + rw
         h1_ptr = base + 2 * rw if silu else None
         ws_ptr = base + (3 if silu else 2) * rw
-        _cabi.check(lib.gca_forward(graph.handle, x.data_ptr(), ldx, w_down.data_ptr(), b_down.data_ptr(),
-                                    w_up.data_ptr(), b_up.data_ptr(), _ptr(scalar), act, int(skip), ws_ptr,
-                                    zp_ptr, h1_ptr, h2_ptr, y.data_ptr(), y.stride(0), d, r, stream), "gca_forward")
+        if addend is None:
+            _cabi.check(lib.gca_forward(graph.handle, x.data_ptr(), ldx, w_down.data_ptr(), b_down.data_ptr(),
+                                        w_up.data_ptr(), b_up.data_ptr(), _ptr(scalar), act, int(skip), ws_ptr,
+                                        zp_ptr, h1_ptr, h2_ptr, y.data_ptr(), y.stride(0), d, r, stream), "gca_forward")
+        else:
+            addend, lda = kernel_operand(addend)
+            _cabi.check(lib.gca_forward_add(graph.handle, x.data_ptr(), ldx, w_down.data_ptr(), b_down.data_ptr(),
+                                            w_up.data_ptr(), b_up.data_ptr(), _ptr(scalar), act, int(skip), ws_ptr,
+                                            zp_ptr, h1_ptr, h2_ptr, addend.data_ptr(), lda, y.data_ptr(), y.stride(0), d, r,
+                                            stream), "gca_forward_add")
+        ctx.has_addend = addend is not None
         ctx.graph, ctx.act, ctx.skip = graph, act, skip
         ctx.has_scalar = scalar is not None
         ctx.silu, ctx.rw = silu, rw
@@ -140,6 +150,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
         n, d = x.shape
         r = w_down.shape[0]
         dev = x.device
+        g_y_in = g_y
         g_y, ldg = kernel_operand(g_y)
         stream = _raw_stream(dev)
         rw = ctx.rw
@@ -147,6 +158,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
         zp_ptr, h2_ptr = base, base + rw
         h1_ptr = base + 2 * rw if ctx.silu else None
         need_x = ctx.needs_input_grad[0]
+        g_a = g_y_in if ctx.has_addend and ctx.needs_input_grad[9] else None     # d(Y + A) / dA = identity
         g_x = torch.empty((n, d), dtype=torch.float32, device=dev) if need_x else None
         # one fresh (non-view) tensor per parameter gradient, so autograd's AccumulateGrad can take ownership
         # of it instead of cloning
@@ -161,7 +173,7 @@ class _GConvAdapterFunction(torch.autograd.Function):
                                      b_up.data_ptr(), _ptr(scalar), ctx.act, int(ctx.skip), ws.data_ptr(),
                                      _ptr(g_x), g_x.stride(0) if need_x else d, g_wd.data_ptr(), g_bd.data_ptr(),
                                      g_wu.data_ptr(), g_bu.data_ptr(), _ptr(g_s), d, r, stream), "gca_backward")
-        return g_x, g_wd, g_bd, g_wu, g_bu, g_s, None, None, None
+        return g_x, g_wd, g_bd, g_wu, g_bu, g_s, None, None, None, g_a
 
 
 class _LayerNormScaleFunction(torch.autograd.Function):
@@ -169,7 +181,8 @@ class _LayerNormScaleFunction(torch.autograd.Function):
     pass backward over ``[N, d]`` (gca_layernorm.cu) instead of the stock LayerNorm + mul kernels."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, scalar, eps: float):
+    def forward(ctx, x, weight, bias, scalar, eps: float, addend=None):
+        """``addend`` (optional, [n, d] fp32): + addend in the same pass (gca_layernorm_scale_add_fwd); its gradient is gY."""
         lib = _cabi.load()
         x, ldx = kernel_operand(x)
         n, d = x.shape
@@ -179,9 +192,16 @@ class _LayerNormScaleFunction(torch.autograd.Function):
         stats = torch.empty((2, max(n, 1)), dtype=torch.float32, device=dev)
         weight = weight.contiguous() if weight is not None else None
         bias = bias.contiguous() if bias is not None else None
-        _cabi.check(lib.gca_layernorm_scale_fwd(x.data_ptr(), ldx, _ptr(weight), _ptr(bias), _ptr(scalar), float(eps),
-                                                y.data_ptr(), y.stride(0), stats[0].data_ptr(), stats[1].data_ptr(), n, d,
-                                                stream), "gca_layernorm_scale_fwd")
+        if addend is None:
+            _cabi.check(lib.gca_layernorm_scale_fwd(x.data_ptr(), ldx, _ptr(weight), _ptr(bias), _ptr(scalar), float(eps),
+                                                    y.data_ptr(), y.stride(0), stats[0].data_ptr(), stats[1].data_ptr(), n, d,
+                                                    stream), "gca_layernorm_scale_fwd")
+        else:
+            addend, lda = kernel_operand(addend)
+            _cabi.check(lib.gca_layernorm_scale_add_fwd(x.data_ptr(), ldx, _ptr(weight), _ptr(bias), _ptr(scalar), float(eps),
+                                                        addend.data_ptr(), lda, y.data_ptr(), y.stride(0), stats[0].data_ptr(),
+                                                        stats[1].data_ptr(), n, d, stream), "gca_layernorm_scale_add_fwd")
+        ctx.has_addend = addend is not None
         ctx.has = (weight is not None, bias is not None, scalar is not None)
         ctx.save_for_backward(x, stats, *[t for t in (weight, bias, scalar) if t is not None])
         return y
@@ -197,6 +217,7 @@ class _LayerNormScaleFunction(torch.autograd.Function):
         scalar = rest.pop(0) if ctx.has[2] else None
         n, d = x.shape
         dev = x.device
+        g_a = g_y if ctx.has_addend and ctx.needs_input_grad[5] else None       # d(Y + A) / dA = identity
         g_y, ldg = kernel_operand(g_y)
         stream = _raw_stream(dev)
         g_x = torch.empty((n, d), dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
@@ -208,7 +229,7 @@ class _LayerNormScaleFunction(torch.autograd.Function):
                                                 _ptr(bias), _ptr(scalar), stats[0].data_ptr(), stats[1].data_ptr(), _ptr(g_x),
                                                 g_x.stride(0) if g_x is not None else d, _ptr(g_w), _ptr(g_b), _ptr(g_s),
                                                 ws.data_ptr(), n, d, stream), "gca_layernorm_scale_bwd")
-        return g_x, g_w, g_b, g_s, None
+        return g_x, g_w, g_b, g_s, None, g_a
 
 
 class _Lin(nn.Module):
@@ -334,15 +355,45 @@ class GConvAdapter(nn.Module):
     def graph_for(self, edge_index: torch.Tensor, num_nodes: int) -> GraphStructure:
         return self.graph_cache.get(edge_index, num_nodes, self.normalize, validate=self.validate_edge_index)
 
-    def forward(self, x: torch.Tensor, edge_index: torch.Tensor, edge_attr: torch.Tensor = None) -> torch.Tensor:
+    def _ln_fused(self, d: int) -> bool:
+        """normalization='layer_norm' runs as the fused LayerNorm + scalar kernels (else as stock torch ops)."""
+        ln = self.normalization
+        return (self.fuse_layer_norm and d % 4 == 0 and d <= 1024 and tuple(ln.normalized_shape) == (d,)
+                and os.environ.get("GCA_DISABLE_LN_FUSE", "0") != "1")
+
+    def fuses_add(self, x: torch.Tensor, h) -> bool:
+        """Whether ``forward(x, ..., add_to=h)`` adds ``h`` in the store of its last kernel: ``h`` is an fp32 tensor on
+        x's device with exactly x's (= the output's) shape, the hidden size needs no column padding (d % 4 == 0), and
+        the tail after the adapter is nothing or the fused LayerNorm.  Any row pitch is fine (odd pitches and broadcast
+        strides are copied, as for x).  Otherwise ``h + out`` runs as a stock op, with the same result."""
+        if not isinstance(h, torch.Tensor) or h.dtype != torch.float32 or h.device != x.device or h.shape != x.shape:
+            return False
+        d = x.shape[-1]
+        if d % 4 != 0:
+            return False
+        if self.normalization is None:
+            return True
+        return isinstance(self.normalization, nn.LayerNorm) and self._ln_fused(d)
+
+    def forward(self, x: torch.Tensor, edge_index: torch.Tensor, edge_attr: torch.Tensor = None, *,
+                add_to: Optional[torch.Tensor] = None) -> torch.Tensor:
         """
         Args:
             x: node features ``[N, hidden_size]`` or ``[1, N, hidden_size]`` (fp32, CUDA).
             edge_index: ``[2, num_edges]`` int64, row 0 = source, row 1 = target.
             edge_attr: accepted and ignored, as in the reference (gconv_adapter.py:80,92).
+            add_to: optional ``h``: return ``h + adapter(x)`` (parallel insertion, src/models/inductive/gnn.py:120-124),
+                with the same value, shape, dtype and gradients as that expression.  See ``fuses_add`` for when the
+                add happens inside the last kernel (bitwise the same result as the separate add).
         Returns:
-            A new tensor of the same shape as ``x``.
+            A new tensor of the same shape as ``x`` (of ``h + out``'s shape and dtype with ``add_to``).
         """
+        if add_to is not None and not self.fuses_add(x, add_to):
+            return add_to + self._forward(x, edge_index, edge_attr, None)
+        return self._forward(x, edge_index, edge_attr, add_to)
+
+    def _forward(self, x: torch.Tensor, edge_index: torch.Tensor, edge_attr, addend: Optional[torch.Tensor]) -> torch.Tensor:
+        """The adapter's output (+ ``addend``, which ``fuses_add`` accepted, when given)."""
         if not x.is_cuda:
             raise RuntimeError("gconv_adapter_b200.GConvAdapter runs on CUDA (sm_100a) only; there is no CPU path")
         if x.dtype != torch.float32:
@@ -350,7 +401,8 @@ class GConvAdapter(nn.Module):
         if x.dim() == 3 and x.size(0) != 1:
             # PyG's node_dim = -2: a leading batch dimension shares the graph; the fused normalisation / scalar tail is
             # row-wise (LayerNorm) or per-call (BatchNorm1d rejects 3-D like the reference's does), so slices are independent
-            return torch.stack([self.forward(x[b], edge_index, edge_attr) for b in range(x.size(0))], dim=0)
+            return torch.stack([self._forward(x[b], edge_index, edge_attr, None if addend is None else addend[b])
+                                for b in range(x.size(0))], dim=0)
         if x.dim() == 3:
             x2 = x[0]
         elif x.dim() == 2:
@@ -365,7 +417,10 @@ class GConvAdapter(nn.Module):
             x2 = F.pad(x2, (0, dp - d))
         graph = self.graph_for(edge_index, n)
         fused_scalar = self.scalar if self.normalization is None else None
-        out = _GConvAdapterFunction.apply(x2, wd, bd, wu, bu, fused_scalar, graph, self._act, self.skip_connection)
+        add2 = None if addend is None else (addend[0] if addend.dim() == 3 else addend)
+        # the addend goes where the adapter's output is finished: the last kernel, or the fused LayerNorm after it
+        out = _GConvAdapterFunction.apply(x2, wd, bd, wu, bu, fused_scalar, graph, self._act, self.skip_connection,
+                                          add2 if self.normalization is None else None)
         if dp != d:
             out = out[:, :d]
         if x.dim() == 3:
@@ -378,10 +433,10 @@ class GConvAdapter(nn.Module):
                 out = self.normalization(out)
         elif isinstance(self.normalization, nn.LayerNorm):
             ln = self.normalization
-            if (self.fuse_layer_norm and d % 4 == 0 and d <= 1024 and tuple(ln.normalized_shape) == (d,)
-                    and os.environ.get("GCA_DISABLE_LN_FUSE", "0") != "1"):
+            if self._ln_fused(d):
                 # LayerNorm + scalar in one pass forward / one pass backward (the scalar is part of the kernel)
-                flat = _LayerNormScaleFunction.apply(out.reshape(-1, d), ln.weight, ln.bias, self.scalar, ln.eps)
+                flat = _LayerNormScaleFunction.apply(out.reshape(-1, d), ln.weight, ln.bias, self.scalar, ln.eps,
+                                                     None if add2 is None else add2.reshape(-1, d))
                 return flat.reshape(out.shape)
             out = ln(out)
         if self.normalization is not None and self.scalar is not None:

@@ -101,6 +101,14 @@ class CudaPhases:
                                              bu.data_ptr(), _ptr(scalar), int(skip), h2_local.data_ptr(), y.data_ptr(),
                                              y.stride(0), _ptr(hub), d, r, self._stream(x)), "gca_fwd_hop2_up")
 
+    def fwd_hop2_up_add(self, g, z_full, x, wu, bu, scalar, skip, h2_local, a, y, hub=None):
+        """fwd_hop2_up, then y += a in the same kernel (a: the local rows of the parallel-insertion addend)."""
+        d, r = wu.shape
+        _cabi.check(self.lib.gca_fwd_hop2_up_add(g.handle, z_full.data_ptr(), x.data_ptr(), row_pitch(x), wu.data_ptr(),
+                                                 bu.data_ptr(), _ptr(scalar), int(skip), h2_local.data_ptr(), a.data_ptr(),
+                                                 row_pitch(a), y.data_ptr(), y.stride(0), _ptr(hub), d, r, self._stream(x)),
+                    "gca_fwd_hop2_up_add")
+
     def bwd_scratch(self, d, r, device):
         return torch.empty(self.lib.gca_bwd_scratch_bytes(d, r), dtype=torch.uint8, device=device)
 
@@ -196,7 +204,7 @@ class PeerMemoryComm:
 
 class _PartitionedFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, w_down, b_down, w_up, b_up, scalar, graph, act, skip, num_nodes, comm, backend):
+    def forward(ctx, x, w_down, b_down, w_up, b_up, scalar, graph, act, skip, num_nodes, comm, backend, addend=None):
         world, rank = comm.world, comm.rank
         s = shard_size(num_nodes, world)
         lo = rank * s
@@ -219,7 +227,11 @@ class _PartitionedFunction(torch.autograd.Function):
             backend.fwd_hop1(graph, p_full, b_down, act, z_full[lo:lo + n], h1, hub, push=comm.push("z", lo, r))
         comm.gather(z_full, lo, s)
         if n > 0:
-            backend.fwd_hop2_up(graph, z_full, x, w_up, b_up, scalar, skip, h2, y, hub)
+            if addend is None:
+                backend.fwd_hop2_up(graph, z_full, x, w_up, b_up, scalar, skip, h2, y, hub)
+            else:
+                backend.fwd_hop2_up_add(graph, z_full, x, w_up, b_up, scalar, skip, h2, kernel_operand(addend)[0], y, hub)
+        ctx.has_addend = addend is not None
         ctx.graph, ctx.act, ctx.skip, ctx.comm, ctx.backend = graph, act, skip, comm, backend
         ctx.meta = (world, s, lo, n, d, r)
         ctx.has_scalar, ctx.has_h1 = scalar is not None, h1 is not None
@@ -246,6 +258,7 @@ class _PartitionedFunction(torch.autograd.Function):
         world, s, lo, n, d, r = ctx.meta
         backend, graph, comm = ctx.backend, ctx.graph, ctx.comm
         dev = x.device
+        g_a = g_y if ctx.has_addend and ctx.needs_input_grad[12] else None      # d(Y + A) / dA = identity
         g_y, _ = kernel_operand(g_y)
         bufs = comm.buffers(world * s, r, dev, ("gh2", "gh1"))
         gh2_full, gh1_full = bufs["gh2"], bufs["gh1"]
@@ -274,7 +287,7 @@ class _PartitionedFunction(torch.autograd.Function):
                                  g_s if scalar is not None else None)
         comm.allreduce_(flat)
         return (g_x, g_wd, g_bd, g_wu, g_bu, g_s.clone() if scalar is not None else None,
-                None, None, None, None, None, None)
+                None, None, None, None, None, None, g_a)
 
 
 class _AllReduceGrad(torch.autograd.Function):
@@ -408,7 +421,24 @@ class PartitionedGConvAdapter(GConvAdapter):
             self._comm.close()
         self._comm, self._comm_key = None, None
 
-    def forward(self, x_local: torch.Tensor, edge_index: torch.Tensor, num_nodes: int, edge_attr=None) -> torch.Tensor:
+    def _ln_fused_partitioned(self, x_local: torch.Tensor) -> bool:
+        d = self.hidden_size
+        return x_local.is_cuda and self.fuse_layer_norm and d <= 1024 and tuple(self.normalization.normalized_shape) == (d,)
+
+    def fuses_add(self, x_local: torch.Tensor, h) -> bool:
+        """Whether ``forward(x_local, ..., add_to=h)`` adds the local rows ``h`` inside the last kernel
+        (gca_fwd_hop2_up_add, or the fused LayerNorm): fp32, x_local's device and shape, and a tail that is nothing or the
+        fused LayerNorm.  Otherwise ``h + out`` runs as a stock op."""
+        if not isinstance(h, torch.Tensor) or h.dtype != torch.float32 or h.device != x_local.device or h.shape != x_local.shape:
+            return False
+        if self.normalization is None:
+            return self._backend is not None and hasattr(self._backend, "fwd_hop2_up_add")
+        return isinstance(self.normalization, nn.LayerNorm) and self._ln_fused_partitioned(x_local)
+
+    def forward(self, x_local: torch.Tensor, edge_index: torch.Tensor, num_nodes: int, edge_attr=None, *,
+                add_to: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``add_to``: this rank's rows of ``h``; returns ``h + adapter(x)[rows]`` (parallel insertion), fused where
+        ``fuses_add`` allows."""
         if self._backend is None:
             self._backend = CudaPhases()
         group = self.process_group
@@ -420,11 +450,14 @@ class PartitionedGConvAdapter(GConvAdapter):
             raise RuntimeError("PartitionedGConvAdapter needs hidden % 4 == 0 and bottleneck in {8,16,32,64}")
         graph = self._graph(edge_index, num_nodes, lo, hi)
         comm = self._get_comm(num_nodes, x_local.device)
+        fuse = add_to is not None and self.fuses_add(x_local, add_to)
+        addend = add_to if fuse else None
         x_local, _ = kernel_operand(x_local)
         fused_scalar = self.scalar if self.normalization is None else None
         out = _PartitionedFunction.apply(x_local, self.conv_down.lin.weight, self.conv_down.bias,
                                          self.conv_up.lin.weight, self.conv_up.bias, fused_scalar, graph, self._act,
-                                         self.skip_connection, num_nodes, comm, self._backend)
+                                         self.skip_connection, num_nodes, comm, self._backend,
+                                         addend if self.normalization is None else None)
         if isinstance(self.normalization, nn.LayerNorm):
             ln = self.normalization
             w, b = _AllReduceGrad.apply(ln.weight, group), _AllReduceGrad.apply(ln.bias, group)
@@ -432,9 +465,11 @@ class PartitionedGConvAdapter(GConvAdapter):
             d = self.hidden_size
             if out.is_cuda and self.fuse_layer_norm and d <= 1024 and tuple(ln.normalized_shape) == (d,):
                 from .finetune.gconv_adapter import _LayerNormScaleFunction      # row-local: the fused tail works per shard
-                out = _LayerNormScaleFunction.apply(out, w, b, sc, ln.eps)
+                out = _LayerNormScaleFunction.apply(out, w, b, sc, ln.eps, addend)
             else:
                 out = torch.nn.functional.layer_norm(out, ln.normalized_shape, w, b, ln.eps)
                 if sc is not None:
                     out = out * sc
+        if add_to is not None and not fuse:
+            out = add_to + out
         return out

@@ -160,6 +160,16 @@ int gca_fwd_hop2_up(const gca_graph* g, const float* Zp_full /*[N,r]*/, const fl
                     const float* Wu /*[d,r]*/, const float* bu /*[d]*/, const float* scalar /*[1] or NULL*/,
                     int skip, float* H2_local /*[n,r]*/, float* Y, int64_t ldy, void* hub_scratch,
                     int32_t d, int32_t r, gca_stream_t stream);
+/* Parallel insertion (h + adapter(h) in one pass): the same as gca_fwd_hop2_up, then + A in the store of the same kernel,
+ *   Y = s * (H2 Wu^T + bu [+ X]) + A
+ * with one round-to-nearest fp32 add per element, so Y has the bits of gca_fwd_hop2_up's Y plus A added separately; the
+ * kernel variant is the one gca_fwd_hop2_up picks.  A: [n, d] local rows, pitched like X (lda >= d, multiple of 4, 16 B
+ * aligned); NULL -> GCA_ERR_INVALID_ARG.  Y == A with ldy == lda is allowed (in-place accumulate); any other overlap of A
+ * with Y is undefined.  The backward needs nothing new: the gradient of A is gY. */
+int gca_fwd_hop2_up_add(const gca_graph* g, const float* Zp_full /*[N,r]*/, const float* X, int64_t ldx,
+                        const float* Wu /*[d,r]*/, const float* bu /*[d]*/, const float* scalar /*[1] or NULL*/,
+                        int skip, float* H2_local /*[n,r]*/, const float* A, int64_t lda, float* Y, int64_t ldy,
+                        void* hub_scratch, int32_t d, int32_t r, gca_stream_t stream);
 
 /* -------- backward phases (autograd of the above) -------- */
 size_t gca_bwd_scratch_bytes(int32_t d, int32_t r);
@@ -201,6 +211,13 @@ int gca_forward(const gca_graph* g, const float* X, int64_t ldx,
                 int act, int skip, void* workspace,
                 float* Zp_save, float* H1_save /*NULL unless silu*/, float* H2_save,
                 float* Y, int64_t ldy, int32_t d, int32_t r, gca_stream_t stream);
+/* gca_forward, then + A (rules of gca_fwd_hop2_up_add): the small-graph cooperative kernel or the phases, whichever
+ * gca_forward would run, with the add in the store of the last one.  Y == A with ldy == lda is allowed. */
+int gca_forward_add(const gca_graph* g, const float* X, int64_t ldx,
+                    const float* Wd, const float* bd, const float* Wu, const float* bu, const float* scalar,
+                    int act, int skip, void* workspace,
+                    float* Zp_save, float* H1_save /*NULL unless silu*/, float* H2_save,
+                    const float* A, int64_t lda, float* Y, int64_t ldy, int32_t d, int32_t r, gca_stream_t stream);
 size_t gca_backward_workspace_bytes(const gca_graph* g, int32_t d, int32_t r);  /* gH2', gH1', gP + partial sums + hub scratch */
 int gca_backward(const gca_graph* g, const float* gY, int64_t ldg, const float* X, int64_t ldx,
                  const float* Zp_save, const float* H1_save, const float* H2_save,
@@ -239,6 +256,11 @@ size_t gca_layernorm_scratch_bytes(int32_t d);
 int    gca_layernorm_scale_fwd(const float* X, int64_t ldx, const float* gamma, const float* beta, const float* scalar,
                                float eps, float* Y, int64_t ldy, float* mean, float* rstd, int32_t n, int32_t d,
                                gca_stream_t stream);
+/* Y = s * LayerNorm(X) + A (parallel insertion with the layer_norm tail; rules for A as in gca_fwd_hop2_up_add, Y == A with
+ * ldy == lda allowed).  mean / rstd as gca_layernorm_scale_fwd writes them; the backward is gca_layernorm_scale_bwd. */
+int    gca_layernorm_scale_add_fwd(const float* X, int64_t ldx, const float* gamma, const float* beta, const float* scalar,
+                                   float eps, const float* A, int64_t lda, float* Y, int64_t ldy, float* mean, float* rstd,
+                                   int32_t n, int32_t d, gca_stream_t stream);
 int    gca_layernorm_scale_bwd(const float* gY, int64_t ldg, const float* X, int64_t ldx, const float* gamma, const float* beta,
                                const float* scalar, const float* mean, const float* rstd, float* gX, int64_t ldgx,
                                float* ggamma, float* gbeta, float* gscalar, void* scratch, int32_t n, int32_t d,
