@@ -62,6 +62,7 @@ SIGNATURES = {
     "gca_graph_get_view": (C.c_int, [_f, C.POINTER(GraphView)]),
     "gca_graph_edge_coef": (C.c_int, [_f, _f, _f]),
     "gca_hub_scratch_bytes": (_sz, [_f]),
+    "gca_hub_scratch_bytes_r": (_sz, [_f, _i32]),
     "gca_propagate": (C.c_int, [_f, C.c_int, _f, _i64, _f, _i64, _f, _f, _i32, _f]),
     "gca_fwd_project": (C.c_int, [_f, _f, _i64, _f, _f, C.POINTER(Push), _i32, _i32, _f]),
     "gca_fwd_hop1": (C.c_int, [_f, _f, _f, C.c_int, _f, _f, _f, C.POINTER(Push), _i32, _f]),

@@ -10,6 +10,10 @@ extern "C" int gca_shape_is_fast(int32_t d, int32_t r) { return shape_ok(d, r) ?
 
 extern "C" size_t gca_hub_scratch_bytes(const gca_graph* g) { return g ? hub_scratch_bytes(g) : 0; }
 
+extern "C" size_t gca_hub_scratch_bytes_r(const gca_graph* g, int32_t r) {
+    return g && r > 0 && r <= 128 ? hub_scratch_bytes(g, r) : 0;
+}
+
 namespace {
 inline bool hub_scratch_ok(const gca_graph* g, const void* hub_scratch) {
     return hub_scratch_bytes(g) == 0 || (hub_scratch && (reinterpret_cast<uintptr_t>(hub_scratch) % kAlign) == 0);
@@ -211,7 +215,7 @@ inline size_t rw_bytes(int n, int r) { return align_up(sizeof(float) * (size_t)(
 extern "C" size_t gca_forward_workspace_bytes(const gca_graph* g, int32_t d, int32_t r) {
     (void)d;
     if (!g || r <= 0) return 0;
-    return rw_bytes(g->row_end - g->row_begin, r) + hub_scratch_bytes(g);
+    return rw_bytes(g->row_end - g->row_begin, r) + hub_scratch_bytes(g, r);
 }
 
 namespace {
@@ -224,7 +228,7 @@ int forward(const gca_graph* g, const float* X, int64_t ldx, const float* Wd, co
     if ((reinterpret_cast<uintptr_t>(workspace) % kAlign) != 0) return GCA_ERR_WORKSPACE;
     char* b = static_cast<char*>(workspace);
     float* Pp = reinterpret_cast<float*>(b);
-    void* hub = hub_scratch_bytes(g) ? b + rw_bytes(g->N, r) : nullptr;
+    void* hub = hub_scratch_bytes(g, r) ? b + rw_bytes(g->N, r) : nullptr;
     // small graphs: one cooperative kernel for the whole forward (anything it cannot take goes through the phases,
     // which also report argument errors)
     if (X && Wd && bd && Wu && bu && Zp_save && H2_save && Y && ldx >= d && ldy >= d && act >= GCA_ACT_NONE &&
@@ -256,7 +260,7 @@ extern "C" int gca_forward_add(const gca_graph* g, const float* X, int64_t ldx, 
 
 extern "C" size_t gca_backward_workspace_bytes(const gca_graph* g, int32_t d, int32_t r) {
     if (!g || d <= 0 || r <= 0) return 0;
-    return 3 * rw_bytes(g->row_end - g->row_begin, r) + gca_bwd_scratch_bytes(d, r) + hub_scratch_bytes(g);
+    return 3 * rw_bytes(g->row_end - g->row_begin, r) + gca_bwd_scratch_bytes(d, r) + hub_scratch_bytes(g, r);
 }
 
 extern "C" int gca_backward(const gca_graph* g, const float* gY, int64_t ldg, const float* X, int64_t ldx,
@@ -273,7 +277,7 @@ extern "C" int gca_backward(const gca_graph* g, const float* gY, int64_t ldg, co
     float* gH1p = reinterpret_cast<float*>(b + rw);
     float* gP = reinterpret_cast<float*>(b + 2 * rw);
     void* scratch = b + 3 * rw;
-    void* hub = hub_scratch_bytes(g) ? b + 3 * rw + gca_bwd_scratch_bytes(d, r) : nullptr;
+    void* hub = hub_scratch_bytes(g, r) ? b + 3 * rw + gca_bwd_scratch_bytes(d, r) : nullptr;
     if (gY && X && Zp_save && H2_save && Wd && Wu && bu && ldg >= d && ldx >= d && (!gX || ldgx >= d) && act >= GCA_ACT_NONE &&
         act <= GCA_ACT_SILU && (act != GCA_ACT_SILU || H1_save) && small_path_ok(g, d, r, static_cast<cudaStream_t>(stream)))
         return small_backward(g, gY, ldg, X, ldx, Zp_save, H1_save, H2_save, Wd, Wu, bu, scalar, act, skip, gH2p, gH1p, gP, gX,

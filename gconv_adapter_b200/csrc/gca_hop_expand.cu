@@ -3,7 +3,8 @@
 // Y = h + adapter(x) in the same pass; gca_fwd_hop2_up_add):
 //   k_hop_expand_tc    tcgen05 / TMEM accumulator, tensor-map TMA in and out, 128-row tiles  (r = 16 / 32, d % 64 == 0, d <= 256)
 //   k_hop_expand_mma   3xTF32 mma.sync, one kernel per 64-row tile                           (r = 16 / 32, other d)
-//   k_hop_expand       FFMA                                                                   (every other shape)
+//   k_hop_expand       FFMA                                                                   (every other shape; r = 128
+//                      after a plain hop, by 128-column blocks: PRE)
 // Reference semantics: /root/reference/src/finetune/gconv_adapter.py:92-106.
 #include "gca_common.cuh"
 #include "gca_device.cuh"
@@ -22,8 +23,13 @@ constexpr int kTileRows = 64;     // rows per CTA tile in k_hop_expand / k_hop_e
 //     Out[i, :] = alpha * (H[i] W + bias) + beta * Resid[i, :]
 // W is kept transposed in shared memory as WT[c][k] so a warp reads 512 contiguous bytes per c.
 // Warp w owns rows 8w..8w+7 of the tile, lane l the column quads l, l+32, ...
+// PRE (r = 128, where all of W next to the H tile would leave one CTA per SM, or not fit from d = 340): H was left in Hout
+// by a plain hop (k_hop, plain mode) and is only read back; the CTA expands the kPreCols output columns of block
+// blockIdx.y, so W^T is held kPreCols columns at a time at every d.
 // ------------------------------------------------------------------------------------------
-template <int R, bool W_IS_DR, bool ADD>
+constexpr int kPreCols = 128;
+
+template <int R, bool W_IS_DR, bool ADD, bool PRE = false>
 __global__ void __launch_bounds__(256, 2)
 k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, const float* __restrict__ dis,
              const float* __restrict__ F, const float* __restrict__ W, const float* __restrict__ bias,
@@ -33,12 +39,28 @@ k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
     const int* __restrict__ hubitem, const float* __restrict__ hub_part, const float* addend, int64_t lda) {
     constexpr int LPG = R / 4, GPW = 32 / LPG;
     extern __shared__ __align__(16) float smem[];
-    float* WT = smem;                 // [R][d]
-    float* Hs = smem + (size_t)R * d; // [kTileRows][R]
-    if (Out) {
-        for (int idx = threadIdx.x; idx < d * R; idx += blockDim.x) {
-            if (W_IS_DR) { const int k = idx / R, c = idx - k * R; WT[c * d + k] = W[idx]; }
-            else WT[idx] = W[idx];
+    float* WT = smem;                 // [R][d]   (PRE: [R][dw], columns col0 .. col0 + dw - 1)
+    float* Hs;                        // [kTileRows][R]
+    int dw = d;
+    if constexpr (PRE) {
+        const int col0 = blockIdx.y * kPreCols;
+        dw = min(kPreCols, d - col0);
+        Hs = smem + (size_t)R * kPreCols;
+        for (int idx = threadIdx.x; idx < dw * R; idx += blockDim.x) {
+            const int c = idx / dw, k = idx - c * dw;
+            WT[idx] = W_IS_DR ? W[(size_t)(col0 + k) * R + c] : W[(size_t)c * d + col0 + k];
+        }
+        bias = bias ? bias + col0 : nullptr;
+        resid = resid ? resid + col0 : nullptr;
+        Out += col0;
+        if constexpr (ADD) addend += col0;
+    } else {
+        Hs = smem + (size_t)R * d;
+        if (Out) {
+            for (int idx = threadIdx.x; idx < d * R; idx += blockDim.x) {
+                if (W_IS_DR) { const int k = idx / R, c = idx - k * R; WT[c * d + k] = W[idx]; }
+                else WT[idx] = W[idx];
+            }
         }
     }
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -46,11 +68,18 @@ k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
     const float s = scalar ? __ldg(scalar) : 1.f;
     const float alpha = alpha_is_scalar ? s : 1.f;
     const float beta = use_resid ? s : 0.f;
-    const int nq = d >> 2;
+    const int nq = dw >> 2;
     const int ntiles = (n + kTileRows - 1) / kTileRows;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int trow = tile * kTileRows;
         __syncthreads();              // WT ready / previous tile's readers of Hs are done
+        if constexpr (PRE) {
+            for (int idx = threadIdx.x; idx < kTileRows * (R / 4); idx += blockDim.x) {
+                const int rr = idx / (R / 4);
+                reinterpret_cast<float4*>(Hs)[idx] =
+                    trow + rr < n ? ldg4(Hout + (size_t)trow * R + (size_t)idx * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        } else
         for (int rr = warp * GPW; rr < kTileRows; rr += 8 * GPW) {
             const int row = trow + rr + grp;
             const bool valid = row < n;
@@ -78,10 +107,10 @@ k_hop_expand(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
             for (int i = 0; i < 8; ++i) acc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
             for (int c4 = 0; c4 < R / 4; ++c4) {
-                const float4 w0 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 0) * d + q * 4);
-                const float4 w1 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 1) * d + q * 4);
-                const float4 w2 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 2) * d + q * 4);
-                const float4 w3 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 3) * d + q * 4);
+                const float4 w0 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 0) * dw + q * 4);
+                const float4 w1 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 1) * dw + q * 4);
+                const float4 w2 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 2) * dw + q * 4);
+                const float4 w3 = *reinterpret_cast<const float4*>(WT + (c4 * 4 + 3) * dw + q * 4);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                     const float4 h = *reinterpret_cast<const float4*>(hs + i * R + c4 * 4);
@@ -686,11 +715,10 @@ k_hop_expand_tc(const int* __restrict__ rowptr, const int* __restrict__ colidx, 
 }
 
 template <int R, bool W_IS_DR, bool ADD>
-int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
-                        const float* bias, const float* resid, int64_t ldr, const float* scalar, int alpha_is_scalar,
-                        int use_resid, float* Hout, float* Out, int64_t ldo, int n, int d, const float* addend, int64_t lda,
-                        cudaStream_t st) {
-    if (n == 0) return GCA_OK;
+int launch_hop_expand_fused_t(const Csr& c, const float* F, const float* W,
+                              const float* bias, const float* resid, int64_t ldr, const float* scalar, int alpha_is_scalar,
+                              int use_resid, float* Hout, float* Out, int64_t ldo, int n, int d, const float* addend, int64_t lda,
+                              cudaStream_t st) {
     GCA_TRY(launch_hub_partials(R, c, F, st));
     const int* rowptr = c.rowptr; const int* colidx = c.colidx; const float* dis = c.dis;
     if constexpr (R == 16 || R == 32) {
@@ -754,6 +782,46 @@ int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
     }
     GCA_LAUNCH_OK();
     return GCA_OK;
+}
+
+// r = 128: the hop as its own kernel (k_hop, plain mode: H -> Hout), then the FFMA expansion of H by column blocks of
+// kPreCols (k_hop_expand<128, ., ., PRE>, blockIdx.y = block).  H has the bits of the fused kernels' H (the same gather).
+template <bool W_IS_DR, bool ADD>
+int launch_hop_expand_wide(const Csr& c, const float* F, const float* W, const float* bias, const float* resid, int64_t ldr,
+                           const float* scalar, int alpha_is_scalar, int use_resid, float* Hout, float* Out, int64_t ldo, int n,
+                           int d, const float* addend, int64_t lda, cudaStream_t st) {
+    constexpr int R = 128;
+    GCA_TRY(launch_hop(R, false, c, F, nullptr, GCA_ACT_NONE, nullptr, nullptr, Hout, nullptr, nullptr, nullptr, n, st, 1,
+                       W_IS_DR ? "hop_plain_fwd" : "hop_plain_bwd"));
+    if (!Out) return GCA_OK;
+    const size_t smem = sizeof(float) * ((size_t)R * kPreCols + (size_t)kTileRows * R);   // 96 KB: two CTAs per SM
+    GCA_TRY(set_smem(k_hop_expand<R, W_IS_DR, ADD, true>, smem));
+    const int ncb = (d + kPreCols - 1) / kPreCols;
+    const int ntiles = (n + kTileRows - 1) / kTileRows;
+    int gx = (2 * num_sms() + ncb - 1) / ncb;
+    if (gx > ntiles) gx = ntiles;
+    {
+        ProfScope ps(W_IS_DR ? "expand_fwd" : "expand_bwd", st, "ffma");
+        k_hop_expand<R, W_IS_DR, ADD, true><<<dim3(gx, ncb), 256, smem, st>>>(c.rowptr, c.colidx, c.dis, F, W, bias, resid, ldr,
+                                                                            scalar, alpha_is_scalar, use_resid, Hout, Out, ldo, n,
+                                                                            d, c.hubitem, c.hub_part, addend, lda);
+    }
+    GCA_LAUNCH_OK();
+    return GCA_OK;
+}
+
+template <int R, bool W_IS_DR, bool ADD>
+int launch_hop_expand_t(const Csr& c, const float* F, const float* W,
+                        const float* bias, const float* resid, int64_t ldr, const float* scalar, int alpha_is_scalar,
+                        int use_resid, float* Hout, float* Out, int64_t ldo, int n, int d, const float* addend, int64_t lda,
+                        cudaStream_t st) {
+    if (n == 0) return GCA_OK;
+    if constexpr (R == 128)
+        return launch_hop_expand_wide<W_IS_DR, ADD>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out, ldo,
+                                                    n, d, addend, lda, st);
+    else
+        return launch_hop_expand_fused_t<R, W_IS_DR, ADD>(c, F, W, bias, resid, ldr, scalar, alpha_is_scalar, use_resid, Hout, Out,
+                                                          ldo, n, d, addend, lda, st);
 }
 
 }  // namespace

@@ -59,13 +59,16 @@ inline Csr csr_of(const gca_graph* g, bool transpose, void* hub_scratch) {
     return transpose ? Csr{g->rowptr_t, g->colidx_t, g->dis, g->hubitem_t, g->item_row_t, g->flags + 4, hp, g->nitems_t, g->N}
                      : Csr{g->rowptr, g->colidx, g->dis, g->hubitem, g->item_row, g->flags + 3, hp, g->nitems, g->N};
 }
-// Bytes of hub scratch one call on this handle needs (0 when the validated build found no hub row).
-inline size_t hub_scratch_bytes(const gca_graph* g) {
+// Bytes of hub scratch one call on this handle needs (0 when the validated build found no hub row): hub_cap items of
+// max(r, 64) floats.  Ranks up to 64 share the 64-float size (gca_hub_scratch_bytes); r = 128 needs twice that.
+inline size_t hub_scratch_bytes(const gca_graph* g, int r = 64) {
     if (g->nitems == 0 && g->nitems_t == 0) return 0;
-    return align_up(sizeof(float) * (size_t)g->hub_cap * 64);
+    return align_up(sizeof(float) * (size_t)g->hub_cap * (r > 64 ? r : 64));
 }
 
-inline bool shape_ok(int d, int r) { return d > 0 && (d % 4) == 0 && (r == 8 || r == 16 || r == 32 || r == 64); }
+inline bool shape_ok(int d, int r) {
+    return d > 0 && (d % 4) == 0 && (r == 8 || r == 16 || r == 32 || r == 64 || r == 128);
+}
 
 bool tc_enabled();        // GCA_DISABLE_TC=1 -> CUDA-core (FFMA) kernels everywhere
 bool stream_enabled();    // GCA_DISABLE_STREAM=1 -> register-fed mma.sync kernels instead of the TMA-fed family
@@ -145,6 +148,7 @@ int launch_finalize(const Scratch& S, const float* Wu, const float* bu, const fl
         case 16: { constexpr int R_ = 16; return CALL; }  \
         case 32: { constexpr int R_ = 32; return CALL; }  \
         case 64: { constexpr int R_ = 64; return CALL; }  \
+        case 128: { constexpr int R_ = 128; return CALL; } \
         default: return GCA_ERR_UNSUPPORTED;            \
     }
 

@@ -76,7 +76,7 @@ extern "C" int gca_nccl_available(void) { return nccl().ok ? 1 : 0; }
 
 extern "C" size_t gca_forward_nccl_workspace_bytes(const gca_graph* g, int32_t world, int32_t d, int32_t r) {
     if (!g || world < 1 || d <= 0 || r <= 0) return 0;
-    return 2 * full_bytes(g->N, world, r) + hub_scratch_bytes(g);
+    return 2 * full_bytes(g->N, world, r) + hub_scratch_bytes(g, r);
 }
 
 extern "C" int gca_forward_nccl(const gca_graph* g, void* nccl_comm, int32_t world, int32_t rank, const float* X, int64_t ldx,
@@ -94,7 +94,7 @@ extern "C" int gca_forward_nccl(const gca_graph* g, void* nccl_comm, int32_t wor
     char* b = static_cast<char*>(workspace);
     float* Pfull = reinterpret_cast<float*>(b);
     float* Zfull = reinterpret_cast<float*>(b + fb);
-    void* hub = hub_scratch_bytes(g) ? b + 2 * fb : nullptr;
+    void* hub = hub_scratch_bytes(g, r) ? b + 2 * fb : nullptr;
     GCA_TRY(gca_fwd_project(g, X, ldx, Wd, Pfull + shard * rank, nullptr, d, r, stream));
     GCA_TRY(gather_rows_inplace(nccl_comm, Pfull, g->N, world, rank, r, st));
     GCA_TRY(gca_fwd_hop1(g, Pfull, bd, act, Zfull + shard * rank, H1_save, hub, nullptr, r, stream));
@@ -107,7 +107,7 @@ extern "C" size_t gca_backward_nccl_workspace_bytes(const gca_graph* g, int32_t 
     if (!g || world < 1 || d <= 0 || r <= 0) return 0;
     const int n = g->row_end - g->row_begin;
     const size_t gp = align_up(sizeof(float) * (size_t)(n > 0 ? n + (n & 1) : 2) * r);
-    return 2 * full_bytes(g->N, world, r) + gp + gca_bwd_scratch_bytes(d, r) + hub_scratch_bytes(g);
+    return 2 * full_bytes(g->N, world, r) + gp + gca_bwd_scratch_bytes(d, r) + hub_scratch_bytes(g, r);
 }
 
 extern "C" int gca_backward_nccl(const gca_graph* g, void* nccl_comm, int32_t world, int32_t rank, const float* gY, int64_t ldg,
@@ -129,7 +129,7 @@ extern "C" int gca_backward_nccl(const gca_graph* g, void* nccl_comm, int32_t wo
     float* gH1full = reinterpret_cast<float*>(b + fb);
     float* gP = reinterpret_cast<float*>(b + 2 * fb);
     void* scratch = b + 2 * fb + gpb;
-    void* hub = hub_scratch_bytes(g) ? b + 2 * fb + gpb + gca_bwd_scratch_bytes(d, r) : nullptr;
+    void* hub = hub_scratch_bytes(g, r) ? b + 2 * fb + gpb + gca_bwd_scratch_bytes(d, r) : nullptr;
     GCA_TRY(gca_bwd_up(g, gY, ldg, H2_save, Wu, scalar, gH2full + shard * rank, scratch, nullptr, d, r, stream));
     GCA_TRY(gather_rows_inplace(nccl_comm, gH2full, g->N, world, rank, r, st));
     GCA_TRY(gca_bwd_hop2(g, gH2full, Zp_save, H1_save, act, gH1full + shard * rank, scratch, hub, nullptr, r, stream));

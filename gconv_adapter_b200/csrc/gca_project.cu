@@ -1,6 +1,7 @@
 // K1 projection  [n,d] x [d,R] -> [n,R]   (conv_down.lin ; gH2' = gY Wu), register-fed variants:
 //   k_project_mma   3xTF32 mma.sync, A fragments straight from global memory            (r = 16 / 32, d % 16 == 0)
-//   k_project       FFMA, register-tiled                                                 (every other shape)
+//   k_project       FFMA, register-tiled                                                 (every other shape; r = 128
+//                   as two 64-column blocks, k_project<64, W_IS_RD, 128>)
 // The default for large inputs is the TMA-fed family in gca_stream.cu; tc::k_project_tc (gca_tc_project.cu) is the
 // tcgen05 / TMEM variant used at r = 32.
 // Reference semantics: /root/reference/src/finetune/gconv_adapter.py:92 (the Linear inside each GCNConv).
@@ -18,7 +19,12 @@ namespace {
 // eight k-quads of a quarter warp hit distinct banks.  Partial sums are combined over the eight
 // kq lanes with a transposing butterfly (56 shuffles for 64 values).
 // ------------------------------------------------------------------------------------------
-template <int R, bool W_IS_RD>
+//
+// RW > R (k_project<64, W_IS_RD, 128>, the r = 128 projection): blockIdx.y picks the R-column block of W and of out that
+// the CTA computes; out's rows are RW floats apart, and so are W's when it is stored [d, RW].  Every block reads all of
+// A: at r = 128 the projection is FFMA-bound (2 r = 256 flop per 4-byte element of A against ~9 flop/B of machine
+// balance), so the second read of A costs bandwidth that is spare.
+template <int R, bool W_IS_RD, int RW = R>
 __global__ void __launch_bounds__(256, 2)
 k_project(const float* __restrict__ A, int64_t lda, const float* __restrict__ W, const float* __restrict__ rowscale,
           const float* __restrict__ scalar, float* __restrict__ out, int n, int d) {
@@ -28,10 +34,16 @@ k_project(const float* __restrict__ A, int64_t lda, const float* __restrict__ W,
     extern __shared__ __align__(16) float smem[];
     float* Ws = smem;
     const int nk4 = d >> 2;
+    if constexpr (RW != R) {
+        const int cb = blockIdx.y * R;
+        W += W_IS_RD ? (size_t)cb * d : (size_t)cb;
+        out += cb;
+    }
     for (int idx = threadIdx.x; idx < d * R; idx += blockDim.x) {
         int k, c;
         if (W_IS_RD) { c = idx / d; k = idx - c * d; } else { k = idx / R; c = idx - k * R; }
-        Ws[(k >> 2) * KS + (k & 3) * R + c] = W[idx];
+        if constexpr (RW == R || W_IS_RD) Ws[(k >> 2) * KS + (k & 3) * R + c] = W[idx];
+        else Ws[(k >> 2) * KS + (k & 3) * R + c] = W[(size_t)k * RW + c];
     }
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -94,7 +106,7 @@ k_project(const float* __restrict__ A, int64_t lda, const float* __restrict__ W,
         const int row = row0 + base / R, c0 = base % R;
         if (row < n) {
             const float sc = (rowscale ? __ldg(rowscale + row) : 1.f) * s;
-            float* o = out + (size_t)row * R + c0;
+            float* o = out + (size_t)row * RW + c0;
             *reinterpret_cast<float4*>(o) = make_float4(v[0] * sc, v[1] * sc, v[2] * sc, v[3] * sc);
             *reinterpret_cast<float4*>(o + 4) = make_float4(v[4] * sc, v[5] * sc, v[6] * sc, v[7] * sc);
         }
@@ -222,9 +234,8 @@ k_project_mma(const float* __restrict__ A, int64_t lda, const float* __restrict_
 }
 
 template <int R, bool W_IS_RD>
-int launch_project_t(const float* A, int64_t lda, const float* W, const float* rowscale, const float* scalar,
-                     float* out, int n, int d, cudaStream_t st) {
-    if (n == 0) return GCA_OK;
+int launch_project_narrow_t(const float* A, int64_t lda, const float* W, const float* rowscale, const float* scalar,
+                            float* out, int n, int d, cudaStream_t st) {
     if (tc_enabled()) {
         // Register-fed tensor-core variants (the TMA-fed family of gca_stream.cu is tried first by the callers):
         // r = 32 -> tcgen05 / TMEM kernel (r = 32 doubles the 3xTF32 mma.sync work; 0.69 vs 0.84 ms at products size),
@@ -263,6 +274,35 @@ int launch_project_t(const float* A, int64_t lda, const float* W, const float* r
     }
     GCA_LAUNCH_OK();
     return GCA_OK;
+}
+
+// r = 128: the 64-column blocks of k_project<64, W_IS_RD, 128> as blockIdx.y = 0 / 1
+template <bool W_IS_RD>
+int launch_project_wide(const float* A, int64_t lda, const float* W, const float* rowscale, const float* scalar,
+                        float* out, int n, int d, cudaStream_t st) {
+    constexpr int TILE = 32;                                  // rows per CTA tile of the R = 64 body
+    const size_t smem = sizeof(float) * (size_t)(d / 4) * (4 * 64 + 4);
+    if (smem > 200 * 1024) return GCA_ERR_UNSUPPORTED;
+    GCA_TRY(set_smem(k_project<64, W_IS_RD, 128>, smem));
+    const int ntiles = (n + TILE - 1) / TILE;
+    const int grid = ntiles < num_sms() ? ntiles : num_sms();   // x 2 halves: two CTAs per SM as for R = 64
+    {
+        ProfScope ps(W_IS_RD ? "project_fwd" : "project_bwd", st, "ffma");
+        k_project<64, W_IS_RD, 128><<<dim3(grid, 2), 256, smem, st>>>(A, lda, W, rowscale, scalar, out, n, d);
+    }
+    GCA_LAUNCH_OK();
+    return GCA_OK;
+}
+
+template <int R, bool W_IS_RD>
+int launch_project_t(const float* A, int64_t lda, const float* W, const float* rowscale, const float* scalar,
+                     float* out, int n, int d, cudaStream_t st) {
+    if (n == 0) return GCA_OK;
+    if constexpr (R == 128) {
+        return launch_project_wide<W_IS_RD>(A, lda, W, rowscale, scalar, out, n, d, st);
+    } else {
+        return launch_project_narrow_t<R, W_IS_RD>(A, lda, W, rowscale, scalar, out, n, d, st);
+    }
 }
 
 }  // namespace

@@ -20,6 +20,7 @@
 
 #include <map>
 #include <mutex>
+#include <tuple>
 
 #include "gca_common.cuh"
 #include "gca_device.cuh"
@@ -437,15 +438,17 @@ bool small_enabled() {
     return on;
 }
 
-// co-resident CTAs of a kernel with `smem` dynamic bytes, per (device, kernel)
+// co-resident CTAs of a kernel with `smem` dynamic bytes, per (device, kernel, smem).  The kernel is part of the key:
+// every k_small_fwd<R, ADD> has the same type K, so one cache serves all ranks, and two ranks can ask with the same smem
+// (r 64 / d 128 and r 128 / d 64) while their register counts allow different numbers of CTAs per SM.
 template <typename K>
 int coop_grid_limit(K kernel, size_t smem) {
     static std::mutex mu;
-    static std::map<std::pair<int, size_t>, int> cache;
+    static std::map<std::tuple<int, const void*, size_t>, int> cache;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return 0;
     std::lock_guard<std::mutex> lk(mu);
-    const auto key = std::make_pair(dev, smem);
+    const auto key = std::make_tuple(dev, reinterpret_cast<const void*>(kernel), smem);
     auto it = cache.find(key);
     if (it != cache.end()) return it->second;
     int per_sm = 0;

@@ -24,7 +24,7 @@ import torch.nn.functional as F
 from .. import _cabi
 from ..graphs.csr import GLOBAL_GRAPH_CACHE, GraphCache, GraphStructure
 
-_FAST_RANKS = (8, 16, 32, 64)
+_FAST_RANKS = (8, 16, 32, 64, 128)
 
 # Test hook: when True the autograd function keeps references to the tensors it saved for the
 # backward (scaled activations Z' and H2) in ``LAST_SAVED`` so parity tests can read the ReLU mask.
@@ -337,13 +337,13 @@ class GConvAdapter(nn.Module):
 
     # ------------------------------------------------------------------------------
     def _padded_params(self, d: int, r: int):
-        """Kernels take d % 4 == 0 and r in {8,16,32,64}; other sizes are zero-padded (exact:
+        """Kernels take d % 4 == 0 and r in {8,16,32,64,128}; other sizes are zero-padded (exact:
         padded channels carry 0 through bias 0 and relu/silu/identity, and their gradients are
         dropped by autograd's slice)."""
         dp = (d + 3) // 4 * 4
         rp = next((c for c in _FAST_RANKS if c >= r), None)
         if rp is None:
-            raise RuntimeError(f"gconv_adapter_b200: bottleneck_size {r} > 64 is not supported by the CUDA kernels")
+            raise RuntimeError(f"gconv_adapter_b200: bottleneck_size {r} > {_FAST_RANKS[-1]} is not supported by the CUDA kernels")
         wd, bd, wu, bu = self.conv_down.lin.weight, self.conv_down.bias, self.conv_up.lin.weight, self.conv_up.bias
         if dp != d or rp != r:
             wd = F.pad(wd, (0, dp - d, 0, rp - r))

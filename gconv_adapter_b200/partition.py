@@ -80,9 +80,9 @@ class CudaPhases:
     def build_graph(self, edge_index, num_nodes, normalize, lo, hi):
         return GraphStructure(edge_index, num_nodes, normalize, lo, hi)
 
-    def hub_scratch(self, g, device):
-        """Per-call scratch for the partial sums of hub rows (None when the graph has no row longer than 512)."""
-        nbytes = self.lib.gca_hub_scratch_bytes(g.handle)
+    def hub_scratch(self, g, device, r):
+        """Per-call scratch for the rank-r partial sums of hub rows (None when the graph has no row longer than 512)."""
+        nbytes = self.lib.gca_hub_scratch_bytes_r(g.handle, r)
         return torch.empty(nbytes, dtype=torch.uint8, device=device) if nbytes else None
 
     def fwd_project(self, g, x, wd, out_local, push=None):
@@ -219,7 +219,7 @@ class _PartitionedFunction(torch.autograd.Function):
         h2 = torch.empty((max(n, 1), r), dtype=torch.float32, device=dev)
         h1 = torch.empty((max(n, 1), r), dtype=torch.float32, device=dev) if act == _cabi.ACT["silu"] else None
         y = torch.empty((n, d), dtype=torch.float32, device=dev)
-        hub = backend.hub_scratch(graph, dev) if hasattr(backend, "hub_scratch") else None
+        hub = backend.hub_scratch(graph, dev, r) if hasattr(backend, "hub_scratch") else None
         if n > 0:
             backend.fwd_project(graph, x, w_down, p_full[lo:lo + n], push=comm.push("p", lo, r))
         comm.gather(p_full, lo, s)
@@ -272,7 +272,7 @@ class _PartitionedFunction(torch.autograd.Function):
         g_bu = flat[2 * d * r:2 * d * r + d]
         g_bd = flat[2 * d * r + d:2 * d * r + d + r]
         g_s = flat[2 * d * r + d + r:]
-        hub = backend.hub_scratch(graph, dev) if hasattr(backend, "hub_scratch") else None
+        hub = backend.hub_scratch(graph, dev, r) if hasattr(backend, "hub_scratch") else None
         if n > 0:
             scratch = backend.bwd_scratch(d, r, dev)
             # one pass over gY: gH2' (pushed to the peers row by row) together with the gWu / gbu partial sums
@@ -446,8 +446,8 @@ class PartitionedGConvAdapter(GConvAdapter):
         lo, hi = row_block(num_nodes, world, rank)
         if x_local.shape != (hi - lo, self.hidden_size):
             raise RuntimeError(f"rank {rank} owns rows [{lo}, {hi}); expected x_local of shape {(hi - lo, self.hidden_size)}")
-        if self.hidden_size % 4 != 0 or self.bottleneck_size not in (8, 16, 32, 64):
-            raise RuntimeError("PartitionedGConvAdapter needs hidden % 4 == 0 and bottleneck in {8,16,32,64}")
+        if self.hidden_size % 4 != 0 or self.bottleneck_size not in (8, 16, 32, 64, 128):
+            raise RuntimeError("PartitionedGConvAdapter needs hidden % 4 == 0 and bottleneck in {8,16,32,64,128}")
         graph = self._graph(edge_index, num_nodes, lo, hi)
         comm = self._get_comm(num_nodes, x_local.device)
         fuse = add_to is not None and self.fuses_add(x_local, add_to)

@@ -84,7 +84,8 @@ int         gca_abi_version(void);
 const char* gca_status_string(int status);
 /* cudaGetErrorString of the last CUDA error this library saw on the calling thread (host string). */
 const char* gca_last_cuda_error(void);
-/* 1 if (d, r) is on the vectorised kernels (d % 4 == 0, r in {8,16,32}); 0 = generic kernels. */
+/* 1 if the adapter phases accept (d, r): d > 0, d % 4 == 0 and r in {8, 16, 32, 64, 128}; 0 otherwise (the phases then
+ * return GCA_ERR_UNSUPPORTED; callers zero-pad r up to the next of these ranks). */
 int         gca_shape_is_fast(int32_t d, int32_t r);
 
 /* -------- graph structure (K0) --------
@@ -127,8 +128,11 @@ int    gca_graph_get_view(const gca_graph* g, gca_graph_view* out /* host */);
 int    gca_graph_edge_coef(const gca_graph* g, float* coef, gca_stream_t stream);
 /* Rows with more than 512 neighbours ("hubs") are pre-reduced per work item into per-CALL scratch of this many bytes
  * (256 B aligned), passed as `hub_scratch` to every phase that walks the graph.  0 when the validated build
- * (gca_graph_validate) found no hub row: hub_scratch may then be NULL. */
+ * (gca_graph_validate) found no hub row: hub_scratch may then be NULL.
+ * gca_hub_scratch_bytes covers every r <= 64; gca_hub_scratch_bytes_r is the size for rank r (r = 128 needs twice as
+ * much), 0 for r outside 1..128.  The *_workspace_bytes queries include the size for their r. */
 size_t gca_hub_scratch_bytes(const gca_graph* g);
+size_t gca_hub_scratch_bytes_r(const gca_graph* g, int32_t r);
 
 /* -------- backbone propagation over the same handle (SURVEY section 8f, rank 3) --------
  * out[i, 0:D] = dst_scale[i] * sum_{j in N(i)} src_scale[j] * X[j, 0:D]  for the handle's rows; transpose = 1 is the adjoint
