@@ -94,6 +94,11 @@ SIGNATURES = {
     "gca_layernorm_scale_fwd": (C.c_int, [_f, _i64, _f, _f, _f, C.c_float, _f, _i64, _f, _f, _i32, _i32, _f]),
     "gca_layernorm_scale_add_fwd": (C.c_int, [_f, _i64, _f, _f, _f, C.c_float, _f, _i64, _f, _i64, _f, _f, _i32, _i32, _f]),
     "gca_layernorm_scale_bwd": (C.c_int, [_f, _i64, _f, _i64, _f, _f, _f, _f, _f, _f, _i64, _f, _f, _f, _f, _i32, _i32, _f]),
+    "gca_batchnorm_scratch_bytes": (_sz, [_i32]),
+    "gca_batchnorm_scale_fwd": (C.c_int, [_f, _i64, _f, _f, _f, C.c_float, C.c_int, C.c_float, _f, _f, _f, _i64, _f, _f, _f,
+                                          _i32, _i32, _f]),
+    "gca_batchnorm_scale_bwd": (C.c_int, [_f, _i64, _f, _i64, _f, _f, _f, _f, _f, C.c_int, _f, _i64, _f, _f, _f, _f, _i32, _i32,
+                                          _f]),
     "gca_nccl_available": (C.c_int, []),
     "gca_forward_nccl_workspace_bytes": (_sz, [_f, _i32, _i32, _i32]),
     "gca_forward_nccl": (C.c_int, [_f, _f, _i32, _i32, _f, _i64, _f, _f, _f, _f, _f, C.c_int, C.c_int, _f, _f, _f, _f, _f, _i64,

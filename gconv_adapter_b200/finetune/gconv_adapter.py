@@ -232,6 +232,58 @@ class _LayerNormScaleFunction(torch.autograd.Function):
         return g_x, g_w, g_b, g_s, None, g_a
 
 
+class _BatchNormScaleFunction(torch.autograd.Function):
+    """``BatchNorm1d(x) * scalar`` for a 2-D ``x`` (gconv_adapter.py:98-106 with normalization='batch_norm') as one
+    statistics pass and one normalizing pass forward, one reduce pass and one gX pass backward (gca_batchnorm.cu) instead
+    of the stock BatchNorm + mul kernels.  ``running_mean`` / ``running_var`` (or None) are updated in place when
+    ``training``; without ``training`` they are the statistics used."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, scalar, running_mean, running_var, training: bool, momentum: float, eps: float):
+        lib = _cabi.load()
+        x, ldx = kernel_operand(x)
+        n, d = x.shape
+        dev = x.device
+        stream = _raw_stream(dev)
+        y = torch.empty((n, d), dtype=torch.float32, device=dev)
+        stats = torch.empty((2, d), dtype=torch.float32, device=dev)
+        ws = torch.empty(lib.gca_batchnorm_scratch_bytes(d), dtype=torch.uint8, device=dev)
+        weight = weight.contiguous() if weight is not None else None
+        bias = bias.contiguous() if bias is not None else None
+        _cabi.check(lib.gca_batchnorm_scale_fwd(x.data_ptr(), ldx, _ptr(weight), _ptr(bias), _ptr(scalar), float(eps),
+                                                int(training), float(momentum), _ptr(running_mean), _ptr(running_var),
+                                                y.data_ptr(), y.stride(0), stats[0].data_ptr(), stats[1].data_ptr(),
+                                                ws.data_ptr(), n, d, stream), "gca_batchnorm_scale_fwd")
+        ctx.training = bool(training)
+        ctx.has = (weight is not None, bias is not None, scalar is not None)
+        ctx.save_for_backward(x, stats, *[t for t in (weight, bias, scalar) if t is not None])
+        return y
+
+    @staticmethod
+    def backward(ctx, g_y):
+        lib = _cabi.load()
+        saved = list(ctx.saved_tensors)
+        x, stats = saved[0], saved[1]
+        rest = saved[2:]
+        weight = rest.pop(0) if ctx.has[0] else None
+        bias = rest.pop(0) if ctx.has[1] else None
+        scalar = rest.pop(0) if ctx.has[2] else None
+        n, d = x.shape
+        dev = x.device
+        g_y, ldg = kernel_operand(g_y)
+        stream = _raw_stream(dev)
+        g_x = torch.empty((n, d), dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
+        g_w = torch.empty((d,), dtype=torch.float32, device=dev) if weight is not None else None
+        g_b = torch.empty((d,), dtype=torch.float32, device=dev) if bias is not None else None
+        g_s = torch.empty((1,), dtype=torch.float32, device=dev) if scalar is not None else None
+        ws = torch.empty(lib.gca_batchnorm_scratch_bytes(d), dtype=torch.uint8, device=dev)
+        _cabi.check(lib.gca_batchnorm_scale_bwd(g_y.data_ptr(), ldg, x.data_ptr(), row_pitch(x), _ptr(weight), _ptr(bias),
+                                                _ptr(scalar), stats[0].data_ptr(), stats[1].data_ptr(), int(ctx.training),
+                                                _ptr(g_x), g_x.stride(0) if g_x is not None else d, _ptr(g_w), _ptr(g_b),
+                                                _ptr(g_s), ws.data_ptr(), n, d, stream), "gca_batchnorm_scale_bwd")
+        return g_x, g_w, g_b, g_s, None, None, None, None, None
+
+
 class _Lin(nn.Module):
     """Holds ``lin.weight`` [out, in] exactly where PyG's ``GCNConv.lin`` (bias-free Linear) has it."""
 
@@ -334,6 +386,7 @@ class GConvAdapter(nn.Module):
         # False: never checked (out-of-range ids are then ignored by the build)
         self.validate_edge_index = True
         self.fuse_layer_norm = True       # normalization='layer_norm': LayerNorm + scalar as one fused pass per direction
+        self.fuse_batch_norm = True       # normalization='batch_norm': BatchNorm1d + scalar as the fused kernels
 
     # ------------------------------------------------------------------------------
     def _padded_params(self, d: int, r: int):
@@ -360,6 +413,40 @@ class GConvAdapter(nn.Module):
         ln = self.normalization
         return (self.fuse_layer_norm and d % 4 == 0 and d <= 1024 and tuple(ln.normalized_shape) == (d,)
                 and os.environ.get("GCA_DISABLE_LN_FUSE", "0") != "1")
+
+    def _bn_fused(self, out: torch.Tensor) -> bool:
+        """normalization='batch_norm' on the adapter's output ``out`` runs as the fused BatchNorm1d + scalar kernels: a
+        plain ``nn.BatchNorm1d`` (not a subclass, whose forward may differ) over ``d`` features, a 2-D fp32 ``out`` with
+        more than one row, d % 4 == 0 and fp32 parameters / buffers.  Otherwise the stock ops run.  ``out`` comes from
+        the adapter kernels, so it is on the GPU."""
+        bn = self.normalization
+        if not (self.fuse_batch_norm and type(bn) is nn.BatchNorm1d and out.dim() == 2 and out.dtype == torch.float32):
+            return False
+        n, d = out.shape
+        if n <= 1 or d % 4 != 0 or bn.num_features != d:
+            return False
+        if any(t is not None and t.dtype != torch.float32 for t in (bn.weight, bn.bias, bn.running_mean, bn.running_var)):
+            return False
+        return os.environ.get("GCA_DISABLE_BN_FUSE", "0") != "1"
+
+    def _batch_norm_scale(self, out: torch.Tensor) -> torch.Tensor:
+        """``self.normalization(out) * self.scalar`` through _BatchNormScaleFunction, with the bookkeeping of
+        ``torch.nn.modules.batchnorm._BatchNorm.forward`` (num_batches_tracked, the averaging factor, which statistics and
+        buffers are used); the kernels update the running buffers."""
+        bn = self.normalization
+        factor = 0.0 if bn.momentum is None else bn.momentum
+        if bn.training and bn.track_running_stats:
+            if bn.num_batches_tracked is not None:
+                bn.num_batches_tracked.add_(1)
+                if bn.momentum is None:         # cumulative moving average
+                    factor = 1.0 / float(bn.num_batches_tracked)
+                else:
+                    factor = bn.momentum
+        bn_training = True if bn.training else (bn.running_mean is None and bn.running_var is None)
+        use_buffers = not bn.training or bn.track_running_stats
+        return _BatchNormScaleFunction.apply(out, bn.weight, bn.bias, self.scalar,
+                                             bn.running_mean if use_buffers else None,
+                                             bn.running_var if use_buffers else None, bn_training, factor, bn.eps)
 
     def fuses_add(self, x: torch.Tensor, h) -> bool:
         """Whether ``forward(x, ..., add_to=h)`` adds ``h`` in the store of its last kernel: ``h`` is an fp32 tensor on
@@ -426,10 +513,13 @@ class GConvAdapter(nn.Module):
         if x.dim() == 3:
             out = out.unsqueeze(0)
 
-        # normalisation needs batch / row statistics of the finished sum: stock torch ops,
-        # then the scalar (which is fused into the kernel only when no normalisation sits between)
+        # normalisation needs batch / row statistics of the finished sum: the fused tails or stock torch ops,
+        # then the scalar (which is fused into the adapter kernel only when no normalisation sits between)
         if isinstance(self.normalization, nn.BatchNorm1d):
             if out.size(0) > 1:
+                if self._bn_fused(out):
+                    # BatchNorm1d + scalar: statistics + one pass forward, one reduce + one gX pass backward
+                    return self._batch_norm_scale(out)
                 out = self.normalization(out)
         elif isinstance(self.normalization, nn.LayerNorm):
             ln = self.normalization

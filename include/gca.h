@@ -270,6 +270,28 @@ int    gca_layernorm_scale_bwd(const float* gY, int64_t ldg, const float* X, int
                                float* ggamma, float* gbeta, float* gscalar, void* scratch, int32_t n, int32_t d,
                                gca_stream_t stream);
 
+/* -------- normalization = 'batch_norm' tail (src/finetune/gconv_adapter.py:54-61, 98-106) --------
+ * Y = s * (gamma * (X - mean_col) * rstd_col + beta): torch.nn.BatchNorm1d on a 2-D [n, d] input followed by the adapter's
+ * learnable scalar.  gamma / beta / scalar may be NULL (= 1 / 0 / 1).  mean, rstd: [d] floats written by the forward and
+ * read by the backward.  X is the forward's input (the output of gca_fwd_hop2_up without scalar).  Any d % 4 == 0.
+ * training != 0: batch statistics (biased variance, eps inside the square root), n >= 2; when running_mean and running_var
+ *   are both non-NULL they are updated in place: r = (1 - momentum) r + momentum * stat, with the unbiased variance
+ *   (var * n / (n - 1)) for running_var.  momentum is the factor torch would use (its `1 / num_batches_tracked` included).
+ * training == 0: mean = running_mean, rstd = 1 / sqrt(running_var + eps) (both buffers required); n == 0 is a no-op.
+ * Backward: training as in the forward (the gradient through the batch statistics, or the elementwise eval gradient);
+ * gX (may be NULL), ggamma / gbeta [d] and gscalar [1] (any may be NULL); n == 0 zeroes the parameter gradients.
+ * scratch: gca_batchnorm_scratch_bytes(d) bytes, 256 B aligned, for either call (per-CTA partial sums combined in a fixed
+ * order: no atomics, bitwise reproducible). */
+size_t gca_batchnorm_scratch_bytes(int32_t d);
+int    gca_batchnorm_scale_fwd(const float* X, int64_t ldx, const float* gamma, const float* beta, const float* scalar,
+                               float eps, int training, float momentum, float* running_mean, float* running_var,
+                               float* Y, int64_t ldy, float* mean, float* rstd, void* scratch,
+                               int32_t n, int32_t d, gca_stream_t stream);
+int    gca_batchnorm_scale_bwd(const float* gY, int64_t ldg, const float* X, int64_t ldx, const float* gamma,
+                               const float* beta, const float* scalar, const float* mean, const float* rstd, int training,
+                               float* gX, int64_t ldgx, float* ggamma, float* gbeta, float* gscalar, void* scratch,
+                               int32_t n, int32_t d, gca_stream_t stream);
+
 /* -------- multi-GPU for a client that owns an NCCL communicator (SURVEY.md section 8b) --------
  * The whole partitioned forward / backward of ONE rank: the phases above with an in-place ncclAllGather of each r-wide
  * operand between them and an ncclAllReduce (sum) of the parameter gradients at the end, all on `stream`.
